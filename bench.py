@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path MarkerDetector::detect on B200 (contract: see README / DESIGN.md section 6).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C1|C2|C3|C4|C5|C4s4]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C1|C2|C3|C4|C5|C4s4] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload = BASELINE.json configs[3] ("C4"): synthetic 3840x2160 grey frames, 100 Fiducidal markers each,
@@ -21,6 +21,11 @@ C2 1280x720 board with erosion + BoardDetector pose, C3 1080p x 64 SUBPIX, C5 HR
 
 --impl reference times that CPU oracle port with all host threads on the FIRST frames of the same batch (the
 reference's own C++ cannot be built here: no OpenCV C++ -- DESIGN.md section 3).
+
+--dump-outputs DIR writes, after the timed steps, the markers the last timed step returned for the batch (rank 0's shard) as
+DIR/<name>.npy, float32/float64: frames (frame index), counts (markers per frame), ids, corners [n,4,2], rvec and tvec [n,3]
+(NaN where a marker has no pose), flattened over the markers in frame order.  The frames are generated from fixed seeds, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -35,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
 
 MARKER_SIZE = 0.05
 N_BASE = 8  # distinct rendered scenes; every frame of a batch gets its own noise realisation
@@ -440,6 +446,21 @@ class Workload:
             pending -= 1
         return total
 
+    def last_step_outputs(self, budget=64 << 20):
+        """What the last step of run_steps() handed its caller (ab_fetch_results: a marker count per frame and that many
+        ab_marker records), as float arrays flattened over the markers in frame order.  A batch whose markers could take
+        more than `budget` bytes is represented by a fixed, seeded sample of its frames (`frames` lists them)."""
+        rec = np.ctypeslib.as_array(self._out).reshape(self.B, self.cap)
+        counts = np.ctypeslib.as_array(self._cnt)
+        frames = np.arange(self.B)
+        per_frame = 16 + 88 * self.cap  # frame index and count; id, corners, rvec, tvec of up to cap markers
+        if self.B * per_frame > budget:
+            frames = np.sort(np.random.default_rng(0).choice(self.B, budget // per_frame, replace=False))
+        m = np.concatenate([rec[f, :counts[f]] for f in frames])
+        pose = m["has_pose"][:, None] != 0
+        return {"frames": frames.astype(np.float64), "counts": counts[frames].astype(np.float64), "ids": m["id"].astype(np.float64),
+                "corners": m["corners"].reshape(-1, 4, 2), "rvec": np.where(pose, m["rvec"], np.nan), "tvec": np.where(pose, m["tvec"], np.nan)}
+
     def time_resident(self, steps, warmup, barrier, sampler=None):
         torch = self.torch
         self.run_steps(max(warmup, 3))
@@ -613,10 +634,11 @@ def measure_config(name, args, rank, local, world, torch, dist, full):
         if not parity["ids_exact"]:
             raise SystemExit("parity check against the oracle failed (%s) -- refusing to report a number" % name)
     steps = args.steps if full else max(5, min(args.steps, 20))
-    if B == 1:
-        steps = max(steps, 200)  # single-frame configs: enough calls for a stable latency
+    if B == 1 and not full:
+        steps = max(steps, 200)  # single-frame configs timed on the side: enough calls for a stable latency
     sampler = ClockSampler(local) if (rank == 0 and full) else None
     ms, n_markers, clocks = wl.time_resident(steps, args.warmup, barrier, sampler)
+    outputs = wl.last_step_outputs() if (full and args.dump_outputs) else None
     kms = wl.kernel_ms()
     t = torch.tensor([ms], device=wl.dev, dtype=torch.float64)
     per_rank = [ms]
@@ -627,7 +649,8 @@ def measure_config(name, args, rank, local, world, torch, dist, full):
     ms_total = max(per_rank)
     fps = world * B * steps / (ms_total / 1e3)
     res = {"name": name, "B": B, "steps": steps, "fps": fps, "ms_total": ms_total, "per_rank_ms": per_rank, "kernel_ms": kms,
-           "markers_per_frame": n_markers / (steps * B), "parity": parity, "clocks": clocks, "counters": wl.det.counters(), "wl": wl}
+           "markers_per_frame": n_markers / (steps * B), "parity": parity, "clocks": clocks, "counters": wl.det.counters(), "wl": wl,
+           "outputs": outputs}
     res["wall_ms"] = wl.wall_ms
     e2e = None
     if not args.skip_e2e:
@@ -690,7 +713,12 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--skip-e2e", action="store_true")
     ap.add_argument("--skip-others", action="store_true", help="skip the short timing of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the markers of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU arm computed: use it with --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -713,6 +741,11 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in res.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        log("[bench] outputs of the last timed step written to %s" % args.dump_outputs)
     unbind_cpus()
     peak, peak_src = measured_peaks()
     roofline = roofline_of(res, world, peak, peak_src)
