@@ -73,6 +73,8 @@ SYMBOLS = {
     "ab_refine_candidate_lines": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
     "ab_calculate_extrinsics": (_i, [_vp, _vp, _i, _vp, _vp, _f, _i]),
     "ab_detect_board": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _f, _f, _i, _vp, _vp]),
+    "ab_set_board": (_i, [_vp, _vp, _vp, _vp, _f, _f, _i]),
+    "ab_get_boards": (_i, [_vp, _i, _vp, _vp, _i]),
     "ab_create_marker_image": (_i, [_vp, _i, _i, _i, _vp, _sz, C.POINTER(C.c_int)]),
     "ab_create_board_image": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _sz, C.POINTER(C.c_int), C.POINTER(C.c_int), _vp, _vp, _i,
                                    C.POINTER(C.c_int)]),

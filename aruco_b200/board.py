@@ -1,6 +1,7 @@
 """Mirror of the caller of the hot path: aruco::BoardConfiguration / Board / BoardDetector
 (src/board.h:56-140, src/boarddetector.{h,cpp}) -- SURVEY 8(f) "next" row 1.  The pose arithmetic (stacked
-4*M-point planar solvePnP, reprojection-outlier re-solve, rotateXAxis) runs on the device (ab_detect_board)."""
+4*M-point planar solvePnP, reprojection-outlier re-solve, rotateXAxis) runs on the device: per call on given markers
+(ab_detect_board), or for whole batches as one more kernel of the batch once setParams armed the board (ab_set_board)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -58,13 +59,38 @@ class BoardDetector:
         self._boardDetected = Board()
 
     def setParams(self, bc: BoardConfiguration, camMatrix=None, distCoeff=None, markerSizeMeters: float = -1.0):
+        """Also arms the board on the marker detector's context: its later batches (detect_batch, enqueue_device) run
+        BoardDetector::detect on every frame.  bc None disarms."""
         self._bconf, self._cam, self._markerSize = bc, (camMatrix, distCoeff), float(markerSizeMeters)
+        self._arm()
 
     def setYPerpendicular(self, enable: bool):
         self._setYPerpendicular = bool(enable)
+        if self._bconf is not None:
+            self._arm()
 
     def set_repj_err_thres(self, v: float):
         self.repj_err_thres = float(v)
+        if self._bconf is not None:
+            self._arm()
+
+    def _arm(self):
+        det = self._mdetector
+        if self._bconf is None:
+            det._check(det._lib.ab_set_board(det._h, None, None, None, -1.0, -1.0, 0))
+            return
+        cfg, keep = self._abi_config(self._bconf)
+        Kf, Df = MarkerDetector._cam(*self._cam)
+        p = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None else None
+        det._check(det._lib.ab_set_board(det._h, C.byref(cfg), p(Kf), p(Df), self._markerSize, float(self.repj_err_thres),
+                                         int(self._setYPerpendicular)))
+
+    @staticmethod
+    def _abi_config(BConf: BoardConfiguration):
+        """ab_board_config over contiguous copies of the configuration (returned too: they must outlive the call)."""
+        ids = np.ascontiguousarray(np.array(BConf.ids, np.int32))
+        pts = np.ascontiguousarray(BConf.objPoints.astype(np.float32).reshape(-1))
+        return ab_board_config(len(ids), BConf.mInfoType, ids.ctypes.data, pts.ctypes.data), (ids, pts)
 
     def getMarkerDetector(self) -> MarkerDetector:
         return self._mdetector
@@ -95,20 +121,48 @@ class BoardDetector:
             for j, v in enumerate(np.asarray(m.corners, np.float32).reshape(8)):
                 buf[i].corners[j] = float(v)
             buf[i].ssize = float(m.ssize)
-        ids = np.ascontiguousarray(np.array(BConf.ids, np.int32))
-        pts = np.ascontiguousarray(BConf.objPoints.astype(np.float32).reshape(-1))
-        cfg = ab_board_config(len(ids), BConf.mInfoType, ids.ctypes.data, pts.ctypes.data)
+        cfg, keep = self._abi_config(BConf)
         Kf, Df = MarkerDetector._cam(camMatrix, distCoeff)
         outm = (ab_marker * max(n, 1))()
         res = ab_board()
         p = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None else None
         det._check(det._lib.ab_detect_board(det._h, buf, n, C.byref(cfg), p(Kf), p(Df), float(markerSizeMeters),
                                             float(self.repj_err_thres), int(self._setYPerpendicular), outm, C.byref(res)))
+        return float(res.prob), self._board(res, outm, 0, BConf)
+
+    @staticmethod
+    def _board(res, bm, off, BConf) -> Board:
         board = Board()
         board.conf = BConf
         for i in range(res.n_markers):
-            board.append(Marker(outm[i].id, np.array(outm[i].corners, np.float32).reshape(4, 2), outm[i].ssize))
+            m = bm[off + i]
+            board.append(Marker(m.id, np.array(m.corners, np.float32).reshape(4, 2), m.ssize))
         if res.has_pose:
             board.Rvec = np.array(res.rvec, np.float64)
             board.Tvec = np.array(res.tvec, np.float64)
-        return float(res.prob), board
+        return board
+
+    # ---- batch path: the board stage runs inside the batch (setParams armed it) ---------------------------------------
+    def _boards(self, markers: List[List[Marker]]):
+        """(prob, Board, markers) per frame of the batch just returned by the marker detector."""
+        det = self._mdetector
+        n = len(markers)
+        cap = max([1] + [len(m) for m in markers])
+        res = (ab_board * max(n, 1))()
+        bm = (ab_marker * (max(n, 1) * cap))()
+        det._check(det._lib.ab_get_boards(det._h, n, res, bm, cap))
+        return [(float(res[f].prob), self._board(res[f], bm, f * cap, self._bconf), markers[f]) for f in range(n)]
+
+    def detect_batch(self, frames: np.ndarray):
+        """BoardDetector::detect(const cv::Mat&) (boarddetector.cpp:66-78) over host frames [n,H,W] u8 or [n,H,W,3] BGR:
+        markers without camera, then the armed board on each frame.  Returns [(prob, Board, markers)] per frame."""
+        return self._boards(self._mdetector.detect_batch(frames))
+
+    def enqueue_device(self, dev_ptr: int, width: int, height: int, n_frames: int, row_stride: Optional[int] = None,
+                       frame_stride: Optional[int] = None):
+        """Device-resident frames (two batches may be in flight, see MarkerDetector.enqueue_device); fetch returns them."""
+        self._mdetector.enqueue_device(dev_ptr, width, height, n_frames, row_stride=row_stride, frame_stride=frame_stride)
+
+    def fetch(self, n_frames: int, cap_per_frame: int = 256):
+        """[(prob, Board, markers)] per frame of the oldest enqueued batch."""
+        return self._boards(self._mdetector.fetch(n_frames, cap_per_frame))

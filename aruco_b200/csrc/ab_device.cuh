@@ -84,6 +84,22 @@ struct HrmDict {
     int correction;
 };
 
+// floats of board-stage scratch per marker slot: 4 object points (12) + 4 image points (8), twice (the outlier re-solve)
+constexpr int BOARD_PTS_PER_MARKER = 40;
+
+// an armed BoardConfiguration with its camera (BoardDetector::setParams); d01, mpp and ssize are computed on the host
+struct BoardArgs {
+    const int32_t* ids;    // [n_cfg], device
+    const float* corners;  // [n_cfg][12], device
+    int n_cfg;
+    int pose;              // a camera was given and the configuration has enough information (boarddetector.cpp:117-130)
+    double mpp;            // marker_meter_per_pix (:132-136)
+    float ssize;
+    float repj_err_thres;
+    int set_y_perp;
+    Camera cam;
+};
+
 struct Batch {
     int W, H, B, wpr;
     int n_t;  // threshold images per frame (2*range+1, setThresholdParamRange); bits/thres hold B*n_t virtual frames
@@ -116,6 +132,10 @@ struct Batch {
     unsigned int* n_quads;    // [B]
     unsigned int* n_cands;    // [B]
     unsigned int* n_markers;  // [B]
+    // board stage (k_board_batch), only when a board configuration is armed (boards == nullptr otherwise)
+    ab_board* boards;      // [B]
+    int32_t* board_slots;  // [B][cap_c] marker indices of the matched markers
+    float* board_pts;      // [B][cap_c * BOARD_PTS_PER_MARKER] obj | img | obj2 | img2 of the stacked correspondences
     // parameters
     int min_len, max_len;  // contour length limits (exclusive)
     int S;                 // warp size

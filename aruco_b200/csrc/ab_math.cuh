@@ -6,6 +6,7 @@
 #include <float.h>
 #include <stdint.h>
 #include "ab_trace.cuh"
+#include "../../include/aruco_b200.h"
 
 namespace ab {
 
@@ -1153,6 +1154,34 @@ AB_HD bool solve_pnp_planar_t(const Camera& cam, const float* obj, const float* 
 }
 AB_HD bool solve_pnp_planar(const Camera& cam, const float* obj, const float* img, int N, double* rvec, double* tvec) {
     return solve_pnp_planar_t<PnpSerial>(cam, obj, img, N, rvec, tvec);
+}
+
+
+// BoardDetector::detect's selection (src/boarddetector.cpp:104-111, 132-150): the markers whose id is in the configuration, in
+// detection order (the first configuration entry with that id wins), stacked as 4 object / image correspondences each.
+// obj: 12 * cap floats, img: 8 * cap floats, slots: cap marker indices.  mpp is the configuration's metres per pixel (1 for
+// a configuration in metres), computed once on the host.  Returns the number of matched markers.
+AB_HD int board_select_stack(const ab_marker* ms, int nm, const int32_t* ids, const float* corners, int n_cfg, double mpp, int cap,
+                             float* obj, float* img, int32_t* slots) {
+    int nb = 0;
+    for (int i = 0; i < nm; i++) {
+        int k = -1;
+        for (int j = 0; j < n_cfg; j++)
+            if (ids[j] == ms[i].id) {
+                k = j;
+                break;
+            }
+        if (k < 0) continue;
+        AB_BOUND(nb < cap);
+        slots[nb] = i;
+        for (int p = 0; p < 4; p++) {
+            img[8 * nb + 2 * p] = ms[i].corners[2 * p];
+            img[8 * nb + 2 * p + 1] = ms[i].corners[2 * p + 1];
+            for (int c = 0; c < 3; c++) obj[12 * nb + 3 * p + c] = (float)((double)corners[(size_t)k * 12 + 3 * p + c] * mpp);  // Point3f * double
+        }
+        nb++;
+    }
+    return nb;
 }
 
 }  // namespace ab

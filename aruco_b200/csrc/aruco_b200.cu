@@ -97,7 +97,7 @@ struct ab_context {
     // timing
     bool timing = false;
     cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t kev[12] = {};  // boundaries: threshold|scan|trace|trace_long|emit|polygon|filter|sample|identify|refine|finalize
+    cudaEvent_t kev[13] = {};  // boundaries: threshold|scan|trace|trace_long|emit|polygon|filter|sample|identify|refine|finalize|board
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
     // Two batches in flight: a second, library-owned context (`twin`) carries the second set of per-batch buffers and
     // a private stream, so ab_enqueue_batch_device may be called again before ab_fetch_results and the kernels of
@@ -115,6 +115,26 @@ struct ab_context {
     // capacities the caller chose in ab_reserve (0 = defaults); kept across automatic re-reservations
     int userQ = 0, userC = 0;
     long long userStarts = 0, userPoints = 0;
+    // armed board configuration (ab_set_board): the device arrays belong to the owner; get_twin copies `board` to the twin
+    int32_t* d_board_ids = nullptr;
+    float* d_board_corners = nullptr;
+    BoardArgs board{};
+    bool have_board = false;
+    // per-batch board outputs of k_board_batch, sized maxB x capC by the first batch that runs with a board armed
+    ab_board* d_boards = nullptr;
+    int32_t* d_board_slots = nullptr;
+    float* d_board_pts = nullptr;
+    int board_frames = 0, board_capc = 0;
+    ab_board* h_boards = nullptr;  // pinned staging of fetch_into
+    size_t h_boards_bytes = 0;
+    int32_t* h_board_slots = nullptr;
+    size_t h_board_slots_bytes = 0;
+    // owner side: the boards of the batch last returned by ab_fetch_results / ab_detect_batch(_bgr), all chunks of it
+    bool res_board = false;          // every chunk of that batch ran with a board armed
+    bool res_board_markers = false;  // and its markers were fetched, so that the matched markers are known
+    std::vector<ab_board> res_boards;
+    std::vector<int32_t> res_off;    // [frames + 1]: frame f's matched markers are res_markers[res_off[f] .. res_off[f + 1])
+    std::vector<ab_marker> res_markers;
 };
 
 // RAII device temporary of the secondary entry points: freed on every return path
@@ -189,6 +209,16 @@ static void free_buffers(ab_context* c) {
     F(c->d_hist);
     F(c->d_markers);
     F(c->d_counters);
+    F(c->d_boards);
+    F(c->d_board_slots);
+    F(c->d_board_pts);
+    c->board_frames = c->board_capc = 0;
+    if (c->h_boards) cudaFreeHost(c->h_boards);
+    c->h_boards = nullptr;
+    c->h_boards_bytes = 0;
+    if (c->h_board_slots) cudaFreeHost(c->h_board_slots);
+    c->h_board_slots = nullptr;
+    c->h_board_slots_bytes = 0;
     if (c->h_markers) cudaFreeHost(c->h_markers);
     c->h_markers = nullptr;
     c->h_markers_bytes = 0;
@@ -273,7 +303,7 @@ int ab_create(int device, ab_context** out) {
     if (const char* e = getenv("ARUCO_B200_GRID_LONG")) ctx->grid_long = std::max(1, atoi(e));
     if (const char* e = getenv("ARUCO_B200_TRACE_REC_MB")) ctx->trace_rec_budget = (size_t)std::max(1, atoi(e)) << 20;
     for (int i = 0; i < 6; i++) cudaEventCreate(&ctx->ev[i]);
-    for (int i = 0; i < 12; i++) cudaEventCreate(&ctx->kev[i]);
+    for (int i = 0; i < 13; i++) cudaEventCreate(&ctx->kev[i]);
     for (int i = 0; i < 2; i++) {
         cudaEventCreateWithFlags(&ctx->ev_h2d[i], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&ctx->ev_done[i], cudaEventDisableTiming);
@@ -302,13 +332,15 @@ void ab_destroy(ab_context* ctx) {
         F(ctx->d_dict_ordids);
         F(ctx->d_dict_ordpos);
         F(ctx->d_dict_tree);
+        F(ctx->d_board_ids);
+        F(ctx->d_board_corners);
     }
     if (ctx->ev_in) cudaEventDestroy(ctx->ev_in);
     if (ctx->d_scratch) cudaFree(ctx->d_scratch);
     if (ctx->h_scratch) cudaFreeHost(ctx->h_scratch);
     for (int i = 0; i < 6; i++)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
-    for (int i = 0; i < 12; i++)
+    for (int i = 0; i < 13; i++)
         if (ctx->kev[i]) cudaEventDestroy(ctx->kev[i]);
     for (int i = 0; i < 2; i++) {
         if (ctx->ev_h2d[i]) cudaEventDestroy(ctx->ev_h2d[i]);
@@ -746,6 +778,11 @@ static Batch sub_view(ab_context* ctx, const Batch& w, int f0, int nf, int s) {
     v.n_quads = w.n_quads + f0;
     v.n_cands = w.n_cands + f0;
     v.n_markers = w.n_markers + f0;
+    if (w.boards) {
+        v.boards = w.boards + f0;
+        v.board_slots = w.board_slots + (size_t)f0 * w.cap_c;
+        v.board_pts = w.board_pts + (size_t)f0 * w.cap_c * BOARD_PTS_PER_MARKER;
+    }
     return v;
 }
 
@@ -885,6 +922,31 @@ static int run_sub(ab_context* ctx, Batch b, cudaStream_t st, bool timing, int s
     CK(cudaGetLastError());
     if (timing) cudaEventRecord(ctx->kev[11], st);
     if (timing) cudaEventRecord(ctx->ev[5], st);
+    if (b.boards) {
+        k_board_batch<<<n, 32, 0, st>>>(b, ctx->board);
+        CK(cudaGetLastError());
+    }
+    if (timing) cudaEventRecord(ctx->kev[12], st);
+    return AB_OK;
+}
+
+// board-stage buffers of this slot for the reserved geometry (maxB frames of capC markers)
+static int ensure_board_buffers(ab_context* ctx) {
+    if (ctx->board_frames >= ctx->maxB && ctx->board_capc == ctx->capC) return AB_OK;
+    auto F = [](auto*& p) {
+        if (p) cudaFree(p);
+        p = nullptr;
+    };
+    F(ctx->d_boards);
+    F(ctx->d_board_slots);
+    F(ctx->d_board_pts);
+    ctx->board_frames = ctx->board_capc = 0;
+    const size_t B = (size_t)ctx->maxB, C = (size_t)ctx->capC;
+    CK(cudaMalloc(&ctx->d_boards, B * sizeof(ab_board)));
+    CK(cudaMalloc(&ctx->d_board_slots, B * C * sizeof(int32_t)));
+    CK(cudaMalloc(&ctx->d_board_pts, B * C * BOARD_PTS_PER_MARKER * sizeof(float)));
+    ctx->board_frames = ctx->maxB;
+    ctx->board_capc = ctx->capC;
     return AB_OK;
 }
 
@@ -916,6 +978,12 @@ static int run_batch(ab_context* ctx, const uint8_t* dgrey, size_t row, size_t f
     Batch b;
     fill_batch(ctx, b, dgrey, row, frame, n, K, D, marker_size);
     b.n_t = n_t;
+    if (ctx->have_board) {
+        if (int rc = ensure_board_buffers(ctx)) return rc;
+        b.boards = ctx->d_boards;
+        b.board_slots = ctx->d_board_slots;
+        b.board_pts = ctx->d_board_pts;
+    }
     cudaStream_t st = ctx->stream;
     CK(cudaMemsetAsync(ctx->d_counters, 0, ctx->counters_bytes, st));
     // Sub-batch pipelining: several stages (long border walks, point emission, polygon fit, refinement, pose) are
@@ -978,6 +1046,8 @@ static int get_twin(ab_context* ctx, ab_context** out) {
     t->params = ctx->params;
     t->dict = ctx->dict;  // device pointers owned by `ctx`
     t->have_dict = ctx->have_dict;
+    t->board = ctx->board;  // device arrays owned by `ctx`
+    t->have_board = ctx->have_board;
     t->cb = ctx->cb;
     t->cb_user = ctx->cb_user;
     t->timing = ctx->timing;
@@ -1028,23 +1098,49 @@ int ab_enqueue_batch_device(ab_context* ctx, const uint8_t* dev_frames, int widt
     return enqueue_on_free_slot(ctx, dev_frames, width, height, row_stride, frame_stride, n_frames, K, D, marker_size);
 }
 
+// grow-only pinned host buffer
+extern "C++" template <class T>
+int ensure_pinned(ab_context* ctx, T*& p, size_t& have, size_t need) {
+    if (need <= have) return AB_OK;
+    if (p) cudaFreeHost(p);
+    p = nullptr;
+    have = 0;
+    CK(cudaMallocHost(&p, need));
+    have = need;
+    return AB_OK;
+}
+
+// the owner's record of the boards of the batch being returned: cleared before its first chunk is fetched
+static void reset_board_results(ab_context* ctx) {
+    ctx->res_board = ctx->res_board_markers = true;
+    ctx->res_boards.clear();
+    ctx->res_markers.clear();
+    ctx->res_off.assign(1, 0);
+}
+
 static int fetch_into(ab_context* ctx, ab_marker* out, int cap, int32_t* counts) {
+    ab_context* own = ctx->owner ? ctx->owner : ctx;
+    const bool board_ok = own->res_board;
+    own->res_board = false;  // stays so when this fetch fails
     if (!ctx->have_last) return set_err(ctx, AB_E_STATE, "no batch has been run");
     const Batch& b = ctx->last;
     int n = ctx->last_n;
     cudaStream_t st = ctx->stream;
     int ncopy = std::min(cap, b.cap_c);
-    size_t need = (size_t)n * ncopy * sizeof(ab_marker);
-    if (need > ctx->h_markers_bytes) {
-        if (ctx->h_markers) cudaFreeHost(ctx->h_markers);
-        ctx->h_markers = nullptr;
-        CK(cudaMallocHost(&ctx->h_markers, need));
-        ctx->h_markers_bytes = need;
-    }
+    if (int rc = ensure_pinned(ctx, ctx->h_markers, ctx->h_markers_bytes, (size_t)n * ncopy * sizeof(ab_marker))) return rc;
     CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, ctx->counters_bytes, cudaMemcpyDeviceToHost, st));
     if (out && ncopy > 0)
         CK(cudaMemcpy2DAsync(ctx->h_markers, (size_t)ncopy * sizeof(ab_marker), b.markers, (size_t)b.cap_c * sizeof(ab_marker),
                              (size_t)ncopy * sizeof(ab_marker), n, cudaMemcpyDeviceToHost, st));
+    if (b.boards) {  // the board records and the matched slots (a frame's slots index its markers: < its count <= ncopy)
+        if (int rc = ensure_pinned(ctx, ctx->h_boards, ctx->h_boards_bytes, (size_t)n * sizeof(ab_board))) return rc;
+        CK(cudaMemcpyAsync(ctx->h_boards, b.boards, (size_t)n * sizeof(ab_board), cudaMemcpyDeviceToHost, st));
+        if (out && ncopy > 0) {
+            if (int rc = ensure_pinned(ctx, ctx->h_board_slots, ctx->h_board_slots_bytes, (size_t)n * ncopy * sizeof(int32_t))) return rc;
+            CK(cudaMemcpy2DAsync(ctx->h_board_slots, (size_t)ncopy * sizeof(int32_t), b.board_slots, (size_t)b.cap_c * sizeof(int32_t),
+                                 (size_t)ncopy * sizeof(int32_t), n, cudaMemcpyDeviceToHost, st));
+        }
+    }
     CK(cudaStreamSynchronize(st));
     Counters csum = *(const Counters*)ctx->h_counters;
     for (int s2 = 1; s2 < MAX_SUB; s2++) csum.err |= ((const Counters*)ctx->h_counters)[s2].err;
@@ -1056,6 +1152,20 @@ static int fetch_into(ab_context* ctx, ab_marker* out, int cap, int32_t* counts)
             return set_err(ctx, AB_E_CAPACITY, "frame %d has %u markers but cap_per_frame is %d", f, nm[f], cap);
         if (counts) counts[f] = (int32_t)nm[f];
         if (out) memcpy(out + (size_t)f * cap, ctx->h_markers + (size_t)f * ncopy, sizeof(ab_marker) * std::min<int>(nm[f], ncopy));
+    }
+    if (b.boards && board_ok) {
+        for (int f = 0; f < n; f++) {
+            const ab_board& bd = ctx->h_boards[f];
+            own->res_boards.push_back(bd);
+            for (int i = 0; out && i < bd.n_markers; i++) {
+                ab_marker m = ctx->h_markers[(size_t)f * ncopy + ctx->h_board_slots[(size_t)f * ncopy + i]];
+                m.ssize = bd.ssize;
+                own->res_markers.push_back(m);
+            }
+            own->res_off.push_back((int32_t)own->res_markers.size());
+        }
+        own->res_board = true;
+        own->res_board_markers = own->res_board_markers && out;
     }
     return AB_OK;
 }
@@ -1069,6 +1179,7 @@ static int fetch_oldest(ab_context* ctx, ab_marker* out, int cap, int32_t* count
         ctx->n_pending--;
     }
     ctx->cur = which;
+    reset_board_results(ctx);
     return fetch_into(slot_of(ctx, which), out, cap, counts);
 }
 
@@ -1100,6 +1211,7 @@ static int detect_host(ab_context* ctx, const uint8_t* frames, int width, int he
         return set_err(ctx, AB_E_INVALID, "bad arguments");
     if (ctx->n_pending) return set_err(ctx, AB_E_STATE, "%d enqueued batch(es) not fetched yet", ctx->n_pending);
     cudaSetDevice(ctx->device);
+    reset_board_results(ctx);
     // chunk size: what was reserved for this geometry, else up to 32 frames
     const int n_t = n_thres_images(ctx->params);
     int chunk = (ctx->W == width && ctx->H == height && ctx->maxB >= n_t) ? std::min(ctx->maxB / n_t, n_frames) : std::min(n_frames, 32);
@@ -1328,7 +1440,7 @@ int ab_get_kernel_ms(ab_context* ctx, float* ms, int n) {
     if (!ctx || !ms || !ctx->timing || !ctx->have_last) return set_err(ctx, AB_E_STATE, "timing not enabled");
     cudaSetDevice(ctx->device);
     CK(cudaStreamSynchronize(ctx->stream));
-    for (int i = 0; i < n && i < 11; i++) CK(cudaEventElapsedTime(&ms[i], ctx->kev[i], ctx->kev[i + 1]));
+    for (int i = 0; i < n && i < 12; i++) CK(cudaEventElapsedTime(&ms[i], ctx->kev[i], ctx->kev[i + 1]));
     return AB_OK;
 }
 
@@ -1622,6 +1734,83 @@ int ab_calculate_extrinsics(ab_context* ctx, ab_marker* markers, int n, const fl
     return AB_OK;
 }
 
+// BoardDetector::detect's constants of a configuration (boarddetector.cpp:95-136), computed once on the host: the kernel
+// must not recompute d01 (a contracted sum of products would change its bits)
+static BoardArgs board_args(const ab_board_config* cfg, const float* K, const float* D, float marker_size, float repj_err_thres,
+                            int set_y_perp) {
+    BoardArgs a;
+    memset(&a, 0, sizeof(a));
+    const float* c0 = cfg->corners;
+    double d01 = sqrt((double)(c0[0] - c0[3]) * (c0[0] - c0[3]) + (double)(c0[1] - c0[4]) * (c0[1] - c0[4]) + (double)(c0[2] - c0[5]) * (c0[2] - c0[5]));
+    a.ssize = -1.f;
+    if (cfg->info_type == 0 && marker_size > 0) a.ssize = marker_size;
+    else if (cfg->info_type == 1) a.ssize = (float)d01;
+    a.mpp = cfg->info_type == 0 ? (double)marker_size / d01 : 1.0;  // marker_meter_per_pix (:132-136)
+    const bool enough = (marker_size > 0 && cfg->info_type == 0) || cfg->info_type == 1;
+    a.pose = K && enough ? 1 : 0;
+    const float zeros[5] = {0, 0, 0, 0, 0};
+    a.cam = make_camera(K, D ? D : zeros);
+    a.n_cfg = cfg->n_markers;
+    a.repj_err_thres = repj_err_thres;
+    a.set_y_perp = set_y_perp;
+    return a;
+}
+
+static bool board_config_ok(const ab_board_config* cfg) {
+    return cfg->n_markers > 0 && cfg->n_markers <= AB_BOARD_MAX_MARKERS && cfg->ids && cfg->corners;
+}
+
+int ab_set_board(ab_context* ctx, const ab_board_config* cfg, const float* K, const float* D, float marker_size, float repj_err_thres,
+                 int set_y_perpendicular) {
+    if (!ctx) return AB_E_INVALID;
+    if (ctx->n_pending)  // a batch in flight reads the configuration
+        return set_err(ctx, AB_E_STATE, "ab_set_board: %d batch(es) in flight, fetch them first", ctx->n_pending);
+    if (cfg && !board_config_ok(cfg))
+        return set_err(ctx, AB_E_INVALID, "ab_set_board: need 1..%d markers with ids and corners", AB_BOARD_MAX_MARKERS);
+    cudaSetDevice(ctx->device);
+    auto F = [](auto*& p) {
+        if (p) cudaFree(p);
+        p = nullptr;
+    };
+    ctx->have_board = false;
+    memset(&ctx->board, 0, sizeof(ctx->board));
+    F(ctx->d_board_ids);
+    F(ctx->d_board_corners);
+    if (!cfg) return AB_OK;
+    const size_t n = (size_t)cfg->n_markers;
+    CK(cudaMalloc(&ctx->d_board_ids, n * sizeof(int32_t)));
+    CK(cudaMalloc(&ctx->d_board_corners, n * 12 * sizeof(float)));
+    CK(cudaMemcpyAsync(ctx->d_board_ids, cfg->ids, n * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_board_corners, cfg->corners, n * 12 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));  // the caller's arrays may be freed on return
+    ctx->board = board_args(cfg, K, D, marker_size, repj_err_thres, set_y_perpendicular);
+    ctx->board.ids = ctx->d_board_ids;
+    ctx->board.corners = ctx->d_board_corners;
+    ctx->have_board = true;
+    return AB_OK;
+}
+
+int ab_get_boards(ab_context* ctx, int n_frames, ab_board* boards, ab_marker* board_markers, int cap_per_frame) {
+    if (!ctx || n_frames < 0 || (n_frames > 0 && !boards) || cap_per_frame < 0) return set_err(ctx, AB_E_INVALID, "ab_get_boards: bad arguments");
+    if (!ctx->res_board) return set_err(ctx, AB_E_STATE, "ab_get_boards: the last batch returned ran without a board armed");
+    if (n_frames != (int)ctx->res_boards.size())
+        return set_err(ctx, AB_E_STATE, "ab_get_boards: the last batch returned has %d frames, not %d", (int)ctx->res_boards.size(), n_frames);
+    if (board_markers) {
+        if (!ctx->res_board_markers)
+            return set_err(ctx, AB_E_STATE, "ab_get_boards: the markers of the last batch were not fetched (out == NULL)");
+        for (int f = 0; f < n_frames; f++)
+            if (ctx->res_boards[f].n_markers > cap_per_frame)
+                return set_err(ctx, AB_E_CAPACITY, "frame %d matched %d board markers but cap_per_frame is %d", f, ctx->res_boards[f].n_markers,
+                               cap_per_frame);
+        for (int f = 0; f < n_frames; f++)
+            memcpy(board_markers + (size_t)f * cap_per_frame, ctx->res_markers.data() + ctx->res_off[f],
+                   sizeof(ab_marker) * (size_t)(ctx->res_off[f + 1] - ctx->res_off[f]));
+    }
+    if (n_frames > 0) memcpy(boards, ctx->res_boards.data(), sizeof(ab_board) * (size_t)n_frames);
+    return AB_OK;
+}
+
+// the markers of one frame as a one-frame batch through k_board_batch
 int ab_detect_board(ab_context* ctx, const ab_marker* markers, int n, const ab_board_config* cfg, const float* K, const float* D,
                     float marker_size, float repj_err_thres, int set_y_perp, ab_marker* board_markers, ab_board* out) {
     if (!ctx || !cfg || !out || n < 0 || (n > 0 && !markers)) return set_err(ctx, AB_E_INVALID, "ab_detect_board: bad arguments");
@@ -1629,68 +1818,42 @@ int ab_detect_board(ab_context* ctx, const ab_marker* markers, int n, const ab_b
     if (cfg->n_markers <= 0 || !cfg->ids || !cfg->corners) return set_err(ctx, AB_E_INVALID, "invalid BoardConfig that is empty");
     cudaSetDevice(ctx->device);
     memset(out, 0, sizeof(*out));
-    const float* c0 = cfg->corners;
-    double d01 = sqrt((double)(c0[0] - c0[3]) * (c0[0] - c0[3]) + (double)(c0[1] - c0[4]) * (c0[1] - c0[4]) + (double)(c0[2] - c0[5]) * (c0[2] - c0[5]));
-    float ssize = -1.f;
-    if (cfg->info_type == 0 && marker_size > 0) ssize = marker_size;
-    else if (cfg->info_type == 1) ssize = (float)d01;
-    // markers that belong to the configuration, in detection order (:104-111) -- pure data selection
-    std::vector<float> obj, img;
-    int nb = 0;
-    double mpp = cfg->info_type == 0 ? (double)marker_size / d01 : 1.0;  // marker_meter_per_pix (:132-136)
-    for (int i = 0; i < n; i++) {
-        int k = -1;
-        for (int j = 0; j < cfg->n_markers; j++)
-            if (cfg->ids[j] == markers[i].id) {
-                k = j;
-                break;
-            }
-        if (k < 0) continue;
-        if (board_markers) {
-            board_markers[nb] = markers[i];
-            board_markers[nb].ssize = ssize;
-        }
-        nb++;
-        for (int p = 0; p < 4; p++) {
-            img.push_back(markers[i].corners[2 * p]);
-            img.push_back(markers[i].corners[2 * p + 1]);
-            for (int c = 0; c < 3; c++) obj.push_back((float)((double)cfg->corners[(size_t)k * 12 + 3 * p + c] * mpp));  // Point3f * double
-        }
-    }
-    out->n_markers = nb;
-    out->ssize = ssize;
-    out->prob = (float)nb / (float)cfg->n_markers;
-    bool enough = (marker_size > 0 && cfg->info_type == 0) || cfg->info_type == 1;
-    if (nb == 0 || !K) {
-        out->prob = 0.f;  // "return 0" (:117-118)
-        return AB_OK;
-    }
-    if (!enough) {
-        out->prob = 0.f;
-        return AB_OK;
-    }
-    int N = 4 * nb;
-    // one grow-only scratch block (obj | img | obj2 | img2 | out) and a pinned result slot: no allocation per call
-    const size_t nf3 = sizeof(float) * 3 * (size_t)N, nf2 = sizeof(float) * 2 * (size_t)N;
-    const size_t off_img = (nf3 + 15) & ~(size_t)15, off_obj2 = off_img + ((nf2 + 15) & ~(size_t)15),
-                 off_img2 = off_obj2 + ((nf3 + 15) & ~(size_t)15), off_out = off_img2 + ((nf2 + 15) & ~(size_t)15);
-    int rcs = ensure_scratch(ctx, off_out + 8 * sizeof(double));
-    if (rcs) return rcs;
+    BoardArgs a = board_args(cfg, K, D, marker_size, repj_err_thres, set_y_perp);
+    const int cap = std::max(n, 1);
+    const size_t ncfg = (size_t)cfg->n_markers;
+    // one grow-only scratch block: markers | count | ids | corners | board | slots | points
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t off_n = al(sizeof(ab_marker) * cap), off_ids = off_n + al(sizeof(unsigned)), off_cor = off_ids + al(sizeof(int32_t) * ncfg),
+                 off_board = off_cor + al(sizeof(float) * 12 * ncfg), off_slots = off_board + al(sizeof(ab_board)),
+                 off_pts = off_slots + al(sizeof(int32_t) * cap), total = off_pts + sizeof(float) * BOARD_PTS_PER_MARKER * cap;
+    if (int rc = ensure_scratch(ctx, total)) return rc;
     uint8_t* base = (uint8_t*)ctx->d_scratch;
-    float *d_obj = (float*)base, *d_img = (float*)(base + off_img), *d_obj2 = (float*)(base + off_obj2), *d_img2 = (float*)(base + off_img2);
-    double* d_out = (double*)(base + off_out);
-    CK(cudaMemcpyAsync(d_obj, obj.data(), nf3, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(d_img, img.data(), nf2, cudaMemcpyHostToDevice, ctx->stream));
-    float zeros[5] = {0, 0, 0, 0, 0};
-    k_board_pose<<<1, 32, 0, ctx->stream>>>(d_obj, d_img, N, make_camera(K, D ? D : zeros), repj_err_thres, set_y_perp, d_obj2, d_img2, d_out);
+    Batch b;
+    memset(&b, 0, sizeof(b));
+    b.B = 1;
+    b.cap_c = cap;
+    b.markers = (ab_marker*)base;
+    b.n_markers = (unsigned*)(base + off_n);
+    b.boards = (ab_board*)(base + off_board);
+    b.board_slots = (int32_t*)(base + off_slots);
+    b.board_pts = (float*)(base + off_pts);
+    a.ids = (const int32_t*)(base + off_ids);
+    a.corners = (const float*)(base + off_cor);
+    const unsigned count = (unsigned)n;
+    if (n > 0) CK(cudaMemcpyAsync(b.markers, markers, sizeof(ab_marker) * n, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(b.n_markers, &count, sizeof(count), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(base + off_ids, cfg->ids, sizeof(int32_t) * ncfg, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(base + off_cor, cfg->corners, sizeof(float) * 12 * ncfg, cudaMemcpyHostToDevice, ctx->stream));
+    k_board_batch<<<1, 32, 0, ctx->stream>>>(b, a);
     CK(cudaGetLastError());
-    double* res = ctx->h_scratch;
-    CK(cudaMemcpyAsync(res, d_out, 8 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    std::vector<int32_t> slots(board_markers ? (size_t)n : 0);
+    CK(cudaMemcpyAsync(ctx->h_scratch, b.boards, sizeof(ab_board), cudaMemcpyDeviceToHost, ctx->stream));
+    if (!slots.empty()) CK(cudaMemcpyAsync(slots.data(), b.board_slots, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    out->has_pose = res[6] != 0.;
-    for (int i = 0; i < 3; i++) {
-        out->rvec[i] = res[i];
-        out->tvec[i] = res[3 + i];
+    memcpy(out, ctx->h_scratch, sizeof(*out));
+    for (int i = 0; board_markers && i < out->n_markers; i++) {
+        board_markers[i] = markers[slots[i]];
+        board_markers[i].ssize = out->ssize;
     }
     return AB_OK;
 }

@@ -5,6 +5,7 @@
 //               chain of a marker is ~20 dependent iterations; as part of k_finalize (128-thread CTAs, one per frame) the
 //               256 frames of a batch needed two waves over the 148 SMs at 7 % warp occupancy (ncu r1x: 0.44 ms).  Warp
 //               CTAs put all markers of the batch on the device at once: one chain latency instead of two.
+//   k_board_batch: one warp per frame -- BoardDetector::detect on the frame's markers (when a board is armed).
 #pragma once
 #include "ab_device.cuh"
 
@@ -140,48 +141,69 @@ __global__ void k_extrinsics(ab_marker* m, int n, Camera cam, float size, int se
     m[i].ssize = size;
 }
 
-// BoardDetector::detect pose part (src/boarddetector.cpp:157-199): ONE WARP over the N stacked corners (the point loops run
-// lane-strided with butterfly sums, see PnpWarp; everything else is computed identically by all lanes).
-// out[0..2] = rvec, out[3..5] = tvec, out[6] = ok, out[7] = points used by the final solve
-__global__ void __launch_bounds__(32) k_board_pose(const float* obj, const float* img, int N, Camera cam, float repj_thres, int set_y_perp,
-                                                   float* obj2, float* img2, double* out) {
-    const int lane = threadIdx.x;
+// BoardDetector::detect (src/boarddetector.cpp:90-204) on every frame of a batch: ONE WARP per frame.  Lane 0 selects the
+// frame's markers that belong to the configuration and stacks their corners (board_select_stack); the pose runs over the N
+// stacked corners with the point loops lane-strided and butterfly sums (see PnpWarp), everything else computed identically by
+// all lanes -- so every branch that reaches a shuffle depends only on values all lanes share (nb, a.pose, ok, the inlier count).
+// Writes one ab_board per frame and the marker indices of the matched markers; ab_detect_board runs this kernel as a
+// one-frame batch.
+__global__ void __launch_bounds__(32) k_board_batch(Batch b, BoardArgs a) {
+    const int f = blockIdx.x, lane = threadIdx.x;
+    const int cap = b.cap_c;
+    const int nm = min((int)b.n_markers[f], cap);
+    float* obj = b.board_pts + (size_t)f * cap * BOARD_PTS_PER_MARKER;
+    float* img = obj + 12 * (size_t)cap;
+    float* obj2 = img + 8 * (size_t)cap;
+    float* img2 = obj2 + 12 * (size_t)cap;
+    int nb = 0;
+    if (lane == 0)
+        nb = board_select_stack(b.markers + (size_t)f * cap, nm, a.ids, a.corners, a.n_cfg, a.mpp, cap, obj, img,
+                                b.board_slots + (size_t)f * cap);
+    nb = __shfl_sync(0xFFFFFFFFu, nb, 0);
+    __syncwarp();  // lane 0's stacked points are visible to the warp
     double r[3] = {0, 0, 0}, t[3] = {0, 0, 0};
-    bool ok = solve_pnp_planar_t<PnpWarp>(cam, obj, img, N, r, t);
-    int used = N;
-    if (ok && repj_thres > 0) {
-        double R[9];
-        rodrigues_to_mat(r, R);
-        int m = 0;
-        for (int n = 0; n < N; n++) {  // order-preserving compaction of the inliers: every lane counts, lane 0 writes
-            double X = obj[3 * n], Y = obj[3 * n + 1], Z = obj[3 * n + 2];
-            double x = R[0] * X + R[1] * Y + R[2] * Z + t[0], y = R[3] * X + R[4] * Y + R[5] * Z + t[1], z = R[6] * X + R[7] * Y + R[8] * Z + t[2];
-            z = z ? 1. / z : 1.;
-            double u, v;
-            distort_norm_to_px(cam, x * z, y * z, &u, &v);
-            float du = (float)u - img[2 * n], dv = (float)v - img[2 * n + 1];  // projectPoints writes Point2f
-            float err = (float)sqrt((double)du * du + (double)dv * dv);
-            if (err < repj_thres) {
-                if (lane == 0) {
-                    for (int c = 0; c < 3; c++) obj2[3 * m + c] = obj[3 * n + c];
-                    img2[2 * m] = img[2 * n];
-                    img2[2 * m + 1] = img[2 * n + 1];
+    bool ok = false;
+    if (nb > 0 && a.pose) {
+        const int N = 4 * nb;
+        ok = solve_pnp_planar_t<PnpWarp>(a.cam, obj, img, N, r, t);
+        if (ok && a.repj_err_thres > 0) {  // reprojection-outlier re-solve (:172-194)
+            double R[9];
+            rodrigues_to_mat(r, R);
+            int m = 0;
+            for (int n = 0; n < N; n++) {  // order-preserving compaction of the inliers: every lane counts, lane 0 writes
+                double X = obj[3 * n], Y = obj[3 * n + 1], Z = obj[3 * n + 2];
+                double x = R[0] * X + R[1] * Y + R[2] * Z + t[0], y = R[3] * X + R[4] * Y + R[5] * Z + t[1], z = R[6] * X + R[7] * Y + R[8] * Z + t[2];
+                z = z ? 1. / z : 1.;
+                double u, v;
+                distort_norm_to_px(a.cam, x * z, y * z, &u, &v);
+                float du = (float)u - img[2 * n], dv = (float)v - img[2 * n + 1];  // projectPoints writes Point2f
+                float err = (float)sqrt((double)du * du + (double)dv * dv);
+                if (err < a.repj_err_thres) {
+                    if (lane == 0) {
+                        AB_BOUND(m < 4 * cap);
+                        for (int c = 0; c < 3; c++) obj2[3 * m + c] = obj[3 * n + c];
+                        img2[2 * m] = img[2 * n];
+                        img2[2 * m + 1] = img[2 * n + 1];
+                    }
+                    m++;
                 }
-                m++;
             }
+            __syncwarp();
+            ok = solve_pnp_planar_t<PnpWarp>(a.cam, obj2, img2, m, r, t);
         }
-        __syncwarp();
-        used = m;
-        ok = solve_pnp_planar_t<PnpWarp>(cam, obj2, img2, m, r, t);
+        if (ok && a.set_y_perp) rotate_x_axis(r);
     }
-    if (ok && set_y_perp) rotate_x_axis(r);
     if (lane == 0) {
+        ab_board o;
+        o.n_markers = nb;
+        o.has_pose = ok ? 1 : 0;
+        o.prob = nb > 0 && a.pose ? (float)nb / (float)a.n_cfg : 0.f;  // "return 0" without camera / information (:117-130)
+        o.ssize = a.ssize;
         for (int i = 0; i < 3; i++) {
-            out[i] = r[i];
-            out[3 + i] = t[i];
+            o.rvec[i] = r[i];
+            o.tvec[i] = t[i];
         }
-        out[6] = ok ? 1. : 0.;
-        out[7] = (double)used;
+        b.boards[f] = o;
     }
 }
 

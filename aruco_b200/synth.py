@@ -1,4 +1,4 @@
-"""Seeded synthetic frames for the benchmark/parity configs C3/C4/C5 (SURVEY.md 8(d)).
+"""Seeded synthetic frames for the benchmark/parity configs C3/C4/C5 (SURVEY.md 8(d)) and for batches of board views.
 
 numpy only (no cv2): white canvas, gx x gy grid of markers, one random homography over the whole
 canvas (4 % inset, +-3 % corner jitter), bilinear sampling with white fill, 3x3 Gaussian blur sigma 0.8,
@@ -136,3 +136,77 @@ def camera_for(W: int, H: int):
     K = np.array([[W, 0, W / 2], [0, W, H / 2], [0, 0, 1]], np.float32)
     D = np.zeros(5, np.float32)
     return K, D
+
+
+def warp_board(board: np.ndarray, corners: np.ndarray, n_frames: int, W: int, H: int, seed: int, sigma: float = 1.5,
+               max_tilt_deg: float = 40.0, min_chain: float = 240.0, border: float = 0.03):
+    """n_frames views of a rendered board (u8 image, white background) through the pinhole camera of camera_for(W, H), each
+    with its own seeded pose -- tilt of the board plane up to max_tilt_deg, in-plane rotation up to 20 degrees, the board
+    filling 65-80 % of the frame height -- bilinear sampling with white fill, render_frame's blur and additive Gaussian
+    noise sigma.  corners:
+    the board configuration in pixels, centred on the image centre (createBoardImage), (n, 4, 3).  A pose is redrawn until
+    every board corner lies `border` inside the frame and every marker's 8-connected outline (sum over its sides of
+    max(|dx|, |dy|)) is at least min_chain pixels.  Returns (frames u8 [n_frames, H, W], homographies [n_frames, 3, 3] from
+    board image pixels to frame pixels)."""
+    rng = np.random.default_rng(seed)
+    bh, bw = board.shape
+    K, _ = camera_for(W, H)
+    K = K.astype(np.float64)
+    ctr = np.array([[1, 0, -(bw // 2)], [0, 1, -(bh // 2)], [0, 0, 1]], np.float64)  # image pixel -> centred board coordinate
+    outline = np.array([[0, 0], [bw - 1, 0], [bw - 1, bh - 1], [0, bh - 1]], np.float64)
+    mk = np.asarray(corners, np.float64)[:, :, :2] + np.array([bw // 2, bh // 2], np.float64)
+
+    def project(Hm, p):
+        q = np.concatenate([p, np.ones(p.shape[:-1] + (1,))], axis=-1) @ Hm.T
+        return q[..., :2] / q[..., 2:3]
+
+    frames = np.empty((n_frames, H, W), np.uint8)
+    homs = np.empty((n_frames, 3, 3))
+    board_f = board.astype(np.float32)
+    for f in range(n_frames):
+        for _ in range(1000):
+            tilt, phi = np.radians(rng.uniform(0, max_tilt_deg)), rng.uniform(0, 2 * np.pi)
+            psi = np.radians(rng.uniform(-20, 20))
+            a = np.array([np.cos(phi), np.sin(phi), 0.0])  # in-plane tilt axis (Rodrigues)
+            Ax = np.array([[0, -a[2], a[1]], [a[2], 0, -a[0]], [-a[1], a[0], 0]])
+            Rt = np.eye(3) + np.sin(tilt) * Ax + (1 - np.cos(tilt)) * Ax @ Ax
+            Rz = np.array([[np.cos(psi), -np.sin(psi), 0], [np.sin(psi), np.cos(psi), 0], [0, 0, 1]])
+            R = Rt @ Rz
+            Z = K[0, 0] * bh / (rng.uniform(0.65, 0.8) * H)
+            t = np.array([rng.uniform(-0.12, 0.12) * W * Z / K[0, 0], rng.uniform(-0.06, 0.06) * H * Z / K[0, 0], Z])
+            Hm = K @ np.column_stack([R[:, 0], R[:, 1], t]) @ ctr
+            o = project(Hm, outline)
+            if not ((o[:, 0] >= border * W).all() and (o[:, 0] <= (1 - border) * W).all() and (o[:, 1] >= border * H).all()
+                    and (o[:, 1] <= (1 - border) * H).all()):
+                continue
+            q = project(Hm, mk)
+            d = np.abs(q - np.roll(q, -1, axis=1))
+            if np.max(d, axis=2).sum(axis=1).min() >= min_chain:
+                break
+        else:
+            raise RuntimeError("warp_board: no pose satisfies the constraints")
+        homs[f] = Hm
+        Hi = np.linalg.inv(Hm)
+        xs = np.arange(W, dtype=np.float64)
+        ys = np.arange(H, dtype=np.float64)[:, None]
+        den = Hi[2, 0] * xs[None, :] + Hi[2, 1] * ys + Hi[2, 2]
+        sx = (Hi[0, 0] * xs[None, :] + Hi[0, 1] * ys + Hi[0, 2]) / den
+        sy = (Hi[1, 0] * xs[None, :] + Hi[1, 1] * ys + Hi[1, 2]) / den
+        fx, fy = np.floor(sx), np.floor(sy)
+        ax, ay = (sx - fx).astype(np.float32), (sy - fy).astype(np.float32)
+        ix, iy = fx.astype(np.int64), fy.astype(np.int64)
+        inside = (ix >= 0) & (iy >= 0) & (ix < bw - 1) & (iy < bh - 1)
+        ixc, iyc = np.clip(ix, 0, bw - 2), np.clip(iy, 0, bh - 2)
+        v = (board_f[iyc, ixc] * (1 - ax) * (1 - ay) + board_f[iyc, ixc + 1] * ax * (1 - ay)
+             + board_f[iyc + 1, ixc] * (1 - ax) * ay + board_f[iyc + 1, ixc + 1] * ax * ay)
+        img = np.where(inside, v, np.float32(255))
+        # the 3x3 Gaussian (sigma 0.8) of render_frame: without it erosion breaks the thin threshold outlines of tilted edges
+        g = np.exp(-1.0 / (2 * 0.8 * 0.8))
+        k3 = np.array([g, 1.0, g], np.float32) / np.float32(1 + 2 * g)
+        p = np.pad(img, 1, mode="edge")
+        img = p[:, :-2] * k3[0] + p[:, 1:-1] * k3[1] + p[:, 2:] * k3[2]
+        img = img[:-2] * k3[0] + img[1:-1] * k3[1] + img[2:] * k3[2]
+        if sigma > 0:
+            img = img + rng.normal(0.0, sigma, size=img.shape).astype(np.float32)
+        frames[f] = np.clip(np.rint(img), 0, 255).astype(np.uint8)
+    return frames, homs

@@ -168,6 +168,24 @@ public:
         if (camParams.isValid()) detect(input, detectedMarkers, camParams.CameraMatrix, camParams.Distorsion, markerSizeMeters, setYPerpendicular);
         else detect(input, detectedMarkers, nullptr, nullptr, markerSizeMeters, setYPerpendicular);
     }
+    // n_frames images of first's geometry, frame_stride bytes apart (0: packed), in one batch, without camera; markers[f] of
+    // frame f.  A board armed on this detector's context (BoardDetector::setParams) runs on every frame as well.
+    void detectBatch(const ImageView& first, int n_frames, size_t frame_stride, std::vector<std::vector<Marker>>& markers) {
+        if (first.empty() || (first.channels != 1 && first.channels != 3) || n_frames < 1)
+            throw Exception(AB_E_INVALID, "detectBatch: 8UC1 or 8UC3 images required");
+        const size_t fs = frame_stride ? frame_stride : first.step * first.rows;
+        std::vector<ab_marker> buf((size_t)n_frames * kCap);
+        std::vector<int32_t> n(n_frames);
+        int rc = first.channels == 1
+                     ? ab_detect_batch(h_, first.data, first.cols, first.rows, first.step, fs, n_frames, nullptr, nullptr, -1.f, buf.data(), kCap, n.data())
+                     : ab_detect_batch_bgr(h_, first.data, first.cols, first.rows, first.step, fs, n_frames, nullptr, nullptr, -1.f, buf.data(), kCap, n.data());
+        check(rc);
+        markers.assign(n_frames, std::vector<Marker>());
+        for (int f = 0; f < n_frames; f++)
+            for (int i = 0; i < n[f]; i++) markers[f].push_back(convert(buf[(size_t)f * kCap + i]));
+        last_rows_ = first.rows;
+        last_cols_ = first.cols;
+    }
 
     // every setter validates a COPY of the parameters and commits it only when the library accepts it (a rejected value
     // must not poison later calls)
@@ -264,6 +282,15 @@ public:
         for (int k = 0; k < 4; k++) candidate[k] = Point2f(c[2 * k], c[2 * k + 1]);
     }
     ab_context* handle() { return h_; }
+    static Marker convert(const ab_marker& m) {
+        Marker r;
+        r.id = m.id;
+        for (int k = 0; k < 4; k++) r.push_back(Point2f(m.corners[2 * k], m.corners[2 * k + 1]));
+        r.ssize = m.ssize;
+        r.hasPose = m.has_pose != 0;
+        for (int k = 0; k < 3; k++) { r.Rvec[k] = m.rvec[k]; r.Tvec[k] = m.tvec[k]; }
+        return r;
+    }
 
 private:
     static const int kCap = 512;
@@ -298,15 +325,6 @@ private:
         check(ab_set_params(h_, &o.p_));
         p_ = o.p_;
         speed_ = o.speed_;
-    }
-    static Marker convert(const ab_marker& m) {
-        Marker r;
-        r.id = m.id;
-        for (int k = 0; k < 4; k++) r.push_back(Point2f(m.corners[2 * k], m.corners[2 * k + 1]));
-        r.ssize = m.ssize;
-        r.hasPose = m.has_pose != 0;
-        for (int k = 0; k < 3; k++) { r.Rvec[k] = m.rvec[k]; r.Tvec[k] = m.tvec[k]; }
-        return r;
     }
 };
 

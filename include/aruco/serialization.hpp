@@ -8,6 +8,7 @@
 // without a space inside flow maps, `!!opencv-matrix`, quoted strings, comments); the writers emit text that
 // cv::FileStorage reads back (tests/test_yaml.py checks both directions against cv2.FileStorage).
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cstdio>
 #include <cstdlib>
@@ -447,9 +448,39 @@ inline Board readBoard(const std::string& path, const std::string& key = "Board"
 class BoardDetector {
 public:
     explicit BoardDetector(MarkerDetector& md, bool setYPerpendicular = false) : md_(md), y_perp_(setYPerpendicular) {}  // boarddetector.h:68
-    void setYPerpendicular(bool enable) { y_perp_ = enable; }   // boarddetector.h:126
+    void setYPerpendicular(bool enable) { y_perp_ = enable; arm(); }   // boarddetector.h:126
     bool isYPerpendicular() const { return y_perp_; }
-    void set_repj_err_thres(float v) { repj_err_thres_ = v; }    // boarddetector.h:134
+    void set_repj_err_thres(float v) { repj_err_thres_ = v; arm(); }    // boarddetector.h:134
+    // setParams (boarddetector.h): the configuration and camera detectBatch uses.  Arms the board on the marker detector's
+    // context, so its batches run BoardDetector::detect on every frame.
+    void setParams(const BoardConfiguration& conf, const CameraParameters& cp, float markerSizeMeters = -1) {
+        conf_ = conf;
+        cp_ = cp;
+        size_ = markerSizeMeters;
+        armed_ = true;
+        arm();
+    }
+    // BoardDetector::detect(const cv::Mat&) (boarddetector.cpp:66-78) over n_frames images of first's geometry, frame_stride
+    // bytes apart (0: packed): markers without camera, then the board of setParams on each frame, in one batch.
+    // Returns the board of every frame; markers[f] receives frame f's markers, prob[f] (when given) the detect return value.
+    std::vector<Board> detectBatch(const ImageView& first, int n_frames, size_t frame_stride, std::vector<std::vector<Marker>>& markers,
+                                   std::vector<float>* prob = nullptr) {
+        if (!armed_) throw Exception(AB_E_STATE, "BoardDetector::detectBatch: setParams first");
+        md_.detectBatch(first, n_frames, frame_stride, markers);
+        size_t cap = 1;
+        for (const auto& m : markers) cap = std::max(cap, m.size());
+        std::vector<ab_board> res(n_frames);
+        std::vector<ab_marker> bm((size_t)n_frames * cap);
+        int rc = ab_get_boards(md_.handle(), n_frames, res.data(), bm.data(), (int)cap);
+        if (rc != AB_OK) throw Exception(rc, ab_last_error(md_.handle()));
+        std::vector<Board> out(n_frames);
+        if (prob) prob->assign(n_frames, 0.f);
+        for (int f = 0; f < n_frames; f++) {
+            fill(out[f], res[f], bm.data() + (size_t)f * cap, conf_);
+            if (prob) (*prob)[f] = res[f].prob;
+        }
+        return out;
+    }
     float get_repj_err_thres() const { return repj_err_thres_; }
     // detect (boarddetector.cpp:90-204): returns the fraction of the board's markers that were found
     float detect(const std::vector<Marker>& detectedMarkers, const BoardConfiguration& conf, Board& out, const CameraParameters& cp,
@@ -478,6 +509,27 @@ public:
         int rc = ab_detect_board(md_.handle(), in.data(), (int)in.size(), &cfg, cam ? cp.CameraMatrix : nullptr, cam ? cp.Distorsion : nullptr,
                                  markerSizeMeters, repj_err_thres_, y_perp_ ? 1 : 0, matched.data(), &res);
         if (rc != AB_OK) throw Exception(rc, ab_last_error(md_.handle()));
+        fill(out, res, matched.data(), conf);
+        return res.prob;
+    }
+
+private:
+    MarkerDetector& md_;
+    bool y_perp_;
+    float repj_err_thres_ = -1;  // boarddetector.cpp:38-41
+    BoardConfiguration conf_;
+    CameraParameters cp_;
+    float size_ = -1;
+    bool armed_ = false;
+    void arm() {
+        if (!armed_) return;
+        const ab_board_config cfg = conf_.abi();
+        const bool cam = cp_.isValid();
+        int rc = ab_set_board(md_.handle(), &cfg, cam ? cp_.CameraMatrix : nullptr, cam ? cp_.Distorsion : nullptr, size_, repj_err_thres_,
+                              y_perp_ ? 1 : 0);
+        if (rc != AB_OK) throw Exception(rc, ab_last_error(md_.handle()));
+    }
+    static void fill(Board& out, const ab_board& res, const ab_marker* matched, const BoardConfiguration& conf) {
         out.clear();
         out.conf = conf;
         out.markerSizeMeters = res.ssize;
@@ -486,25 +538,8 @@ public:
             out.Rvec[k] = res.rvec[k];
             out.Tvec[k] = res.tvec[k];
         }
-        for (int i = 0; i < res.n_markers; i++) {
-            Marker m;
-            m.id = matched[i].id;
-            for (int k = 0; k < 4; k++) m.push_back(Point2f(matched[i].corners[2 * k], matched[i].corners[2 * k + 1]));
-            m.ssize = matched[i].ssize;
-            m.hasPose = matched[i].has_pose != 0;
-            for (int k = 0; k < 3; k++) {
-                m.Rvec[k] = matched[i].rvec[k];
-                m.Tvec[k] = matched[i].tvec[k];
-            }
-            out.push_back(m);
-        }
-        return res.prob;
+        for (int i = 0; i < res.n_markers; i++) out.push_back(MarkerDetector::convert(matched[i]));
     }
-
-private:
-    MarkerDetector& md_;
-    bool y_perp_;
-    float repj_err_thres_ = -1;  // boarddetector.cpp:38-41
 };
 
 // ---- HRM dictionary (src/highlyreliablemarkers.h:95-112) -------------------------------------------------------------

@@ -149,7 +149,7 @@ AB_API int ab_enable_timing(ab_context* ctx, int enable);
 AB_API int ab_get_stage_ms(ab_context* ctx, float* ms, int n);
 /* per-kernel device milliseconds of the last batch: [0]=threshold(+erosion) [1]=scan_starts [2]=trace (short walks)
  * [3]=trace (parked long walks) [4]=emit [5]=polygon [6]=frame_filter [7]=homography + sample (the warp stage)
- * [8]=otsu + identify [9]=refine [10]=finalize(+pose)                                                         */
+ * [8]=otsu + identify [9]=refine [10]=finalize(+pose) [11]=board (k_board_batch; ~0 when no board is armed)     */
 AB_API int ab_get_kernel_ms(ab_context* ctx, float* ms, int n);
 
 /* ---- public workers of MarkerDetector ---------------------------------------------------------------- */
@@ -190,10 +190,28 @@ typedef struct ab_board {
     double tvec[3];
 } ab_board;
 /* id filter, stacked 4*M-point solvePnP, optional reprojection-outlier re-solve (repj_err_thres > 0, cpp:172-194),
- * optional rotateXAxis.  board_markers (cap n) receives the matched markers in input order.                 */
+ * optional rotateXAxis.  board_markers (cap n) receives the matched markers in input order.  Runs the board kernel of the
+ * batch path (ab_set_board) on these markers as a one-frame batch.                                                   */
 AB_API int ab_detect_board(ab_context* ctx, const ab_marker* markers, int n, const ab_board_config* cfg, const float* K,
                            const float* D, float marker_size, float repj_err_thres, int set_y_perpendicular,
                            ab_marker* board_markers, ab_board* out);
+/* largest configuration ab_set_board accepts (a 32 x 32 board) */
+#define AB_BOARD_MAX_MARKERS 1024
+/* BoardDetector::setParams (boarddetector.h) for the batch path: every later ab_enqueue_batch_device / ab_detect_batch /
+ * ab_detect_batch_bgr of this context also runs BoardDetector::detect (boarddetector.cpp:90-204) on each frame's markers, in
+ * one more kernel of the batch whose results come back with the markers.
+ * The configuration is copied (the caller's arrays may be freed on return); K/D/marker_size are the BOARD's camera, independent
+ * of the K/D given to the enqueue (those still govern the marker stage: LINES undistortion, per-marker pose).
+ * cfg == NULL disarms.  AB_E_STATE while a batch is in flight; AB_E_INVALID for an empty configuration, NULL ids / corners
+ * or more than AB_BOARD_MAX_MARKERS markers.                                                                         */
+AB_API int ab_set_board(ab_context* ctx, const ab_board_config* cfg, const float* K, const float* D, float marker_size,
+                        float repj_err_thres, int set_y_perpendicular);
+/* The boards of the batch most recently returned by ab_fetch_results / ab_detect_batch(_bgr): boards[n_frames]; board_markers
+ * (n_frames * cap_per_frame, may be NULL) receives each frame's matched markers in detection order with ssize set -- exactly what
+ * ab_detect_board returns for that frame's markers.  AB_E_STATE if that batch ran without a board armed, n_frames differs, or
+ * board_markers is requested but the markers were not fetched (out == NULL); AB_E_CAPACITY if a frame matched more markers
+ * than cap_per_frame.                                                                                                 */
+AB_API int ab_get_boards(ab_context* ctx, int n_frames, ab_board* boards, ab_marker* board_markers, int cap_per_frame);
 
 /* ---- next row: marker / board rendering on the device ----------------------------------------------------- */
 /* FiducidalMarkers::createMarkerImage (src/arucofidmarkers.cpp:213-263) without the text watermark (cv::putText
