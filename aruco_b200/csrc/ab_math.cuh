@@ -708,14 +708,6 @@ AB_HD bool solve6_spd(const double A[6][6], double* b) {
 }
 
 // corners: 4 x (u,v) f32 in the reference's order; size = marker side; out rvec/tvec f64.
-#if defined(AB_PNP_COUNT) && !defined(__CUDA_ARCH__)
-static int g_pnp_evals = 0, g_pnp_iters = 0;  // host-check instrumentation: residual evaluations / accepted steps of the last solve
-#define AB_PNP_EVAL() (g_pnp_evals++)
-#define AB_PNP_ITER() (g_pnp_iters++)
-#else
-#define AB_PNP_EVAL() ((void)0)
-#define AB_PNP_ITER() ((void)0)
-#endif
 AB_HD bool solve_pnp_marker(const Camera& cam, const float* corners, float size, double* rvec, double* tvec) {
     float h = size / 2.f;  // getObjectPoints, src/marker.cpp:91-108
     float obj[12] = {-h, -h, 0, -h, h, 0, h, h, 0, h, -h, 0};
@@ -818,7 +810,6 @@ AB_HD bool solve_pnp_marker(const Camera& cam, const float* corners, float size,
             }
             for (int i = 0; i < 6; i++) p[i] = prev[i] - d[i];
             // state CHECK_ERR
-            AB_PNP_EVAL();
             pnp_residual(cam, p, obj, m, err);
             double s = 0;
             for (int k = 0; k < 8; k++) s += err[k] * err[k];
@@ -832,7 +823,6 @@ AB_HD bool solve_pnp_marker(const Camera& cam, const float* corners, float size,
             dn += (p[i] - prev[i]) * (p[i] - prev[i]);
             pn += prev[i] * prev[i];
         }
-        AB_PNP_ITER();
         if (++iters >= 20 || sqrt(dn) / sqrt(pn) < FLT_EPSILON) break;
         prevErrNorm = errNorm;
         pnp_residual_jacobian(cam, p, obj, m, err, J);

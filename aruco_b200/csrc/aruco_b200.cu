@@ -24,7 +24,9 @@
 
 using namespace ab;
 
-constexpr int MAX_SUB = 4;  // sub-batches (streams) a batch can be pipelined over
+constexpr int WALKER_CTAS_PER_SM = 8;  // persistent grids of k_trace<false> and k_trace<true>
+// d_counters / h_counters: one Counters, then the per-frame n_quads, n_cands and n_markers arrays (maxB entries each)
+constexpr size_t FRAME_COUNTS_OFFSET = sizeof(Counters);
 
 #ifndef AB_SOURCE_HASH
 #define AB_SOURCE_HASH "unknown"
@@ -40,15 +42,10 @@ struct ab_context {
     cudaStream_t user_stream = nullptr;  // ab_set_stream: the caller's stream; each enqueue is ordered after it
     bool has_user_stream = false;
     cudaStream_t copy_stream = nullptr;
-    cudaStream_t sub_stream[MAX_SUB] = {};
-    cudaEvent_t ev_fork = nullptr, ev_join[MAX_SUB] = {};
-    int n_sub_streams = 1;  // measured on B200: no gain from 2-4 sub-batches (full grids leave no room to co-schedule)
-    int grid_trace = 8, grid_long = 8;  // CTAs per SM of the persistent walker grids
     uint2* d_trace_rec = nullptr;       // strips of k_trace<true>'s lanes (k_contours.cuh), grown on demand
-    size_t trace_rec_bytes = 0, rec_sub_bytes = 0;
+    size_t trace_rec_bytes = 0;
     unsigned rec_ctas = 0, rec_half = 0;
     size_t trace_rec_budget = (size_t)6 << 30;  // more lanes than this pays for are not launched
-    int last_nsub = 1;
     ab_params params;
     std::string err;
     // reserved geometry
@@ -273,11 +270,6 @@ int ab_create(int device, ab_context** out) {
         delete ctx;
         return AB_E_CUDA;
     }
-    for (int i = 0; i < MAX_SUB; i++) {
-        cudaStreamCreateWithFlags(&ctx->sub_stream[i], cudaStreamNonBlocking);
-        cudaEventCreateWithFlags(&ctx->ev_join[i], cudaEventDisableTiming);
-    }
-    cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming);
     {  // step tables of the border walkers (ab_trace.cuh)
         std::vector<uint8_t> lut(2 * WALK_LUT_SIZE);
         for (uint32_t i = 0; i < (uint32_t)WALK_LUT_SIZE; i++) {
@@ -295,12 +287,8 @@ int ab_create(int device, ab_context** out) {
             return AB_E_CUDA;
         }
     }
-    if (const char* e = getenv("ARUCO_B200_SUBBATCHES")) ctx->n_sub_streams = std::max(1, std::min(MAX_SUB, atoi(e)));
-    // walker grids in CTAs per SM (tuning knobs for variant studies)
     // capacity of the parked-walk queue per frame (tests shrink it to exercise the finish-in-place path)
     if (const char* e = getenv("ARUCO_B200_CAP_LONG")) ctx->capLongPF = (unsigned)std::max(1, atoi(e));
-    if (const char* e = getenv("ARUCO_B200_GRID_TRACE")) ctx->grid_trace = std::max(1, atoi(e));
-    if (const char* e = getenv("ARUCO_B200_GRID_LONG")) ctx->grid_long = std::max(1, atoi(e));
     if (const char* e = getenv("ARUCO_B200_TRACE_REC_MB")) ctx->trace_rec_budget = (size_t)std::max(1, atoi(e)) << 20;
     for (int i = 0; i < 6; i++) cudaEventCreate(&ctx->ev[i]);
     for (int i = 0; i < 13; i++) cudaEventCreate(&ctx->kev[i]);
@@ -346,11 +334,6 @@ void ab_destroy(ab_context* ctx) {
         if (ctx->ev_h2d[i]) cudaEventDestroy(ctx->ev_h2d[i]);
         if (ctx->ev_done[i]) cudaEventDestroy(ctx->ev_done[i]);
     }
-    for (int i = 0; i < MAX_SUB; i++) {
-        if (ctx->sub_stream[i]) cudaStreamDestroy(ctx->sub_stream[i]);
-        if (ctx->ev_join[i]) cudaEventDestroy(ctx->ev_join[i]);
-    }
-    if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     delete ctx;
@@ -498,7 +481,7 @@ static int reserve_impl(ab_context* ctx, int width, int height, int max_batch) {
     const int S_alloc = std::max(ctx->params.warp_size, 56);
     const size_t B = (size_t)max_batch;
     const size_t bw = bit_image_words(width, height);
-    const size_t counters_bytes = MAX_SUB * sizeof(Counters) + 3 * B * sizeof(unsigned);
+    const size_t counters_bytes = FRAME_COUNTS_OFFSET + 3 * B * sizeof(unsigned);
     cudaError_t e = cudaSuccess;
     auto A = [&](auto** p, size_t bytes) {
         if (e == cudaSuccess) e = cudaMalloc(p, bytes);
@@ -688,14 +671,16 @@ __global__ void k_bgr2grey(const uint8_t* bgr, size_t row, size_t frame, uint8_t
     }
 }
 
-static int fill_batch(ab_context* ctx, Batch& b, const uint8_t* dgrey, size_t row, size_t frame, int n, const float* K,
+// n frames of n_t threshold images each: the per-frame capacities of the append lists count the n * n_t virtual frames
+static int fill_batch(ab_context* ctx, Batch& b, const uint8_t* dgrey, size_t row, size_t frame, int n, int n_t, const float* K,
                       const float* D, float marker_size) {
     const ab_params& P = ctx->params;
+    const int nv = n * n_t;
     memset(&b, 0, sizeof(b));
     b.W = ctx->W;
     b.H = ctx->H;
     b.B = n;
-    b.n_t = 1;
+    b.n_t = n_t;
     b.wpr = bit_words_per_row(ctx->W);
     b.bits_words = bit_image_words(ctx->W, ctx->H);
     b.grey = dgrey;
@@ -705,14 +690,14 @@ static int fill_batch(ab_context* ctx, Batch& b, const uint8_t* dgrey, size_t ro
     b.bits = ctx->d_bits;
     b.bits2 = ctx->d_bits2;
     b.starts = ctx->d_starts;
-    b.cap_starts = (unsigned long long)ctx->capStartsPF * n;
+    b.cap_starts = (unsigned long long)ctx->capStartsPF * nv;
     b.contours = ctx->d_contours;
-    b.cap_contours = ctx->capContoursPF * (unsigned)n;
+    b.cap_contours = ctx->capContoursPF * (unsigned)nv;
     b.longq = ctx->d_longq;
-    b.cap_long = ctx->capLongPF * (unsigned)n;
+    b.cap_long = ctx->capLongPF * (unsigned)nv;
     b.walk_lut = ctx->d_walk_lut;
     b.pool = ctx->d_pool;
-    b.cap_pool = (unsigned long long)ctx->capPoolPF * n;
+    b.cap_pool = (unsigned long long)ctx->capPoolPF * nv;
     b.quads = ctx->d_quads;
     b.cap_q = ctx->capQ;
     b.cands = ctx->d_cands;
@@ -722,7 +707,7 @@ static int fill_batch(ab_context* ctx, Batch& b, const uint8_t* dgrey, size_t ro
     b.hist = ctx->d_hist;
     b.markers = ctx->d_markers;
     b.cnt = (Counters*)ctx->d_counters;
-    b.n_quads = (unsigned*)(ctx->d_counters + MAX_SUB * sizeof(Counters));
+    b.n_quads = (unsigned*)(ctx->d_counters + FRAME_COUNTS_OFFSET);
     b.n_cands = b.n_quads + ctx->maxB;
     b.n_markers = b.n_cands + ctx->maxB;
     // contour length limits (src/markerdetector.cpp:500-501): f32 product truncated to int
@@ -749,43 +734,6 @@ static int fill_batch(ab_context* ctx, Batch& b, const uint8_t* dgrey, size_t ro
     return AB_OK;
 }
 
-// launches the whole path for frames resident at `dgrey`
-// view of frames [f0, f0+nf) of a batch as sub-batch s: per-frame buffers are offset, the append lists are
-// partitioned by the per-frame capacities, counters are per sub-batch
-static Batch sub_view(ab_context* ctx, const Batch& w, int f0, int nf, int s) {
-    Batch v = w;
-    const size_t vt = (size_t)w.n_t;  // virtual frames per frame
-    v.B = nf;
-    v.grey = w.grey + (size_t)f0 * w.grey_frame;
-    v.thres = w.thres + (size_t)f0 * vt * w.W * w.H;
-    v.bits = w.bits + (size_t)f0 * vt * w.bits_words;
-    v.bits2 = w.bits2 + (size_t)f0 * vt * w.bits_words;
-    v.starts = w.starts + (size_t)ctx->capStartsPF * vt * f0;
-    v.cap_starts = (unsigned long long)ctx->capStartsPF * vt * nf;
-    v.contours = w.contours + (size_t)ctx->capContoursPF * vt * f0;
-    v.cap_contours = ctx->capContoursPF * (unsigned)(vt * nf);
-    v.pool = w.pool + (size_t)ctx->capPoolPF * vt * f0;
-    v.cap_pool = (unsigned long long)ctx->capPoolPF * vt * nf;
-    v.longq = w.longq + (size_t)ctx->capLongPF * vt * f0;
-    v.cap_long = ctx->capLongPF * (unsigned)(vt * nf);
-    v.quads = w.quads + (size_t)f0 * w.cap_q;
-    v.cands = w.cands + (size_t)f0 * w.cap_c;
-    v.canon = w.canon + (size_t)f0 * w.cap_c * (size_t)(w.S * w.S);
-    v.aux = w.aux + (size_t)f0 * w.cap_c;
-    v.hist = w.hist + (size_t)f0 * w.cap_c * 256;
-    v.markers = w.markers + (size_t)f0 * w.cap_c;
-    v.cnt = w.cnt + s;
-    v.n_quads = w.n_quads + f0;
-    v.n_cands = w.n_cands + f0;
-    v.n_markers = w.n_markers + f0;
-    if (w.boards) {
-        v.boards = w.boards + f0;
-        v.board_slots = w.board_slots + (size_t)f0 * w.cap_c;
-        v.board_pts = w.board_pts + (size_t)f0 * w.cap_c * BOARD_PTS_PER_MARKER;
-    }
-    return v;
-}
-
 // LINES refinement; the contour is undistorted first only with a distorted camera (cpp:957-959; all-zero coefficients
 // make cv::undistortPoints the identity on pixel coordinates, see Camera::zero_D)
 static void launch_refine_lines(const Batch& b, cudaStream_t st) {
@@ -795,14 +743,14 @@ static void launch_refine_lines(const Batch& b, cudaStream_t st) {
 }
 
 // k_trace<true>: every lane of the persistent grid owns a strip of max_len / 2 + 2 recorded pixel pairs (30 KB at 4K), so the
-// grid is as large as the parked walks can use, the configured CTAs per SM allow and the strip budget pays for.  Concurrent
-// sub-batches share the grid and the strips evenly.  Called once per batch, before its first launch.
-static int plan_trace_long(ab_context* ctx, int max_len, unsigned cap_long_sub, int nsub) {
+// grid is as large as the parked walks can use, WALKER_CTAS_PER_SM allows and the strip budget pays for.  Called once per
+// batch, before its first launch.
+static int plan_trace_long(ab_context* ctx, int max_len, unsigned cap_long) {
     const size_t half = ((size_t)(std::max(max_len, 0) / 2 + 2) + 1) & ~(size_t)1;  // even: 16-byte aligned strips
-    size_t ctas = (size_t)ctx->sm_count * (size_t)std::max(1, ctx->grid_long / nsub);
-    ctas = std::min(ctas, ((size_t)cap_long_sub + 127) / 128);
-    ctas = std::max<size_t>(1, std::min(ctas, ctx->trace_rec_budget / nsub / (half * 128 * sizeof(uint2))));
-    const size_t sub_bytes = ctas * 128 * half * sizeof(uint2), need = sub_bytes * nsub;
+    size_t ctas = (size_t)ctx->sm_count * WALKER_CTAS_PER_SM;
+    ctas = std::min(ctas, ((size_t)cap_long + 127) / 128);
+    ctas = std::max<size_t>(1, std::min(ctas, ctx->trace_rec_budget / (half * 128 * sizeof(uint2))));
+    const size_t need = ctas * 128 * half * sizeof(uint2);
     if (need > ctx->trace_rec_bytes) {  // grows only when the geometry or the maximum contour size grew
         if (ctx->d_trace_rec) cudaFree(ctx->d_trace_rec);
         ctx->d_trace_rec = nullptr;
@@ -816,20 +764,73 @@ static int plan_trace_long(ab_context* ctx, int max_len, unsigned cap_long_sub, 
     }
     ctx->rec_ctas = (unsigned)ctas;
     ctx->rec_half = (unsigned)half;
-    ctx->rec_sub_bytes = sub_bytes;
     return AB_OK;
 }
-static void launch_trace_long(ab_context* ctx, Batch& bv, cudaStream_t st, int sub) {
-    bv.trace_rec = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(ctx->d_trace_rec) + ctx->rec_sub_bytes * sub);
+static void launch_trace_long(ab_context* ctx, Batch& bv, cudaStream_t st) {
+    bv.trace_rec = ctx->d_trace_rec;
     bv.rec_half = ctx->rec_half;
     k_trace<true><<<ctx->rec_ctas, 128, 0, st>>>(bv);
 }
 
-// one sub-batch (a view of the batch buffers) on one stream: every stage of the path
-static int run_sub(ab_context* ctx, Batch b, cudaStream_t st, bool timing, int sub = 0) {
+// board-stage buffers of this slot for the reserved geometry (maxB frames of capC markers)
+static int ensure_board_buffers(ab_context* ctx) {
+    if (ctx->board_frames >= ctx->maxB && ctx->board_capc == ctx->capC) return AB_OK;
+    auto F = [](auto*& p) {
+        if (p) cudaFree(p);
+        p = nullptr;
+    };
+    F(ctx->d_boards);
+    F(ctx->d_board_slots);
+    F(ctx->d_board_pts);
+    ctx->board_frames = ctx->board_capc = 0;
+    const size_t B = (size_t)ctx->maxB, C = (size_t)ctx->capC;
+    CK(cudaMalloc(&ctx->d_boards, B * sizeof(ab_board)));
+    CK(cudaMalloc(&ctx->d_board_slots, B * C * sizeof(int32_t)));
+    CK(cudaMalloc(&ctx->d_board_pts, B * C * BOARD_PTS_PER_MARKER * sizeof(float)));
+    ctx->board_frames = ctx->maxB;
+    ctx->board_capc = ctx->capC;
+    return AB_OK;
+}
+
+// launches the whole path for frames resident at `dgrey`
+static int run_batch(ab_context* ctx, const uint8_t* dgrey, size_t row, size_t frame, int n, const float* K,
+                     const float* D, float marker_size) {
     const ab_params& P = ctx->params;
-    const int n = b.B, n_t = b.n_t;
+    if (P.decoder == AB_DECODER_HRM && !ctx->have_dict)
+        return set_err(ctx, AB_E_STATE, "HRM decoder selected but no dictionary loaded (ab_load_hrm_dictionary)");
+    if (P.decoder == AB_DECODER_HOST_CALLBACK && !ctx->cb)
+        return set_err(ctx, AB_E_STATE, "host-callback decoder selected but no callback set");
+    if (P.decoder == AB_DECODER_HRM && (ctx->dict.n + 2) > P.warp_size)
+        return set_err(ctx, AB_E_INVALID, "warp size too small for the dictionary");
+    if (P.corner_method == AB_CORNER_SUBPIX && ((int)P.thres_param1 < 1 || (int)P.thres_param1 > 24))
+        return set_err(ctx, AB_E_INVALID, "SUBPIX window %d outside 1..24", (int)P.thres_param1);
+    if (P.locked_corners && ((int)P.thres_param1 < 1 || (int)P.thres_param1 > 24))
+        return set_err(ctx, AB_E_INVALID, "locked-corner window %d outside 1..24", (int)P.thres_param1);
+    // setThresholdParamRange (markerdetector.h:152, cpp:322-334): 2*range+1 threshold images per frame, param1 =
+    // p1 - range + range*i (sic, SURVEY B.6); they live as n_t consecutive "virtual frames" per frame for the
+    // threshold / contour / polygon stages and are merged per frame by k_polygon's quad keys.
+    // CANNY ignores the parameters: the reference's 2r+1 identical edge images yield duplicate candidates that its
+    // too-near filter removes again (cpp:322-334, :592-627), so one image gives the same result.
+    const int n_t = n_thres_images(P);
+    if (n * n_t > ctx->maxB) return set_err(ctx, AB_E_STATE, "internal: %d virtual frames > reserved %d", n * n_t, ctx->maxB);
+    {   // k_scan_starts indexes its work items with 32 bits
+        const unsigned long long items = 8ull * (unsigned long long)((ctx->W + 31) >> 5) * (unsigned long long)((ctx->H + 2 + BIT_TILE - 1) / BIT_TILE) *
+                                         (unsigned long long)(n * n_t);
+        if (items >= (1ull << 32)) return set_err(ctx, AB_E_INVALID, "batch of %d frames %dx%d is too large for one launch: split it", n, ctx->W, ctx->H);
+    }
+    Batch b;
+    fill_batch(ctx, b, dgrey, row, frame, n, n_t, K, D, marker_size);
+    if (ctx->have_board) {
+        if (int rc = ensure_board_buffers(ctx)) return rc;
+        b.boards = ctx->d_boards;
+        b.board_slots = ctx->d_board_slots;
+        b.board_pts = ctx->d_board_pts;
+    }
+    cudaStream_t st = ctx->stream;
+    const bool timing = ctx->timing;
     const int sms = ctx->sm_count;
+    CK(cudaMemsetAsync(ctx->d_counters, 0, ctx->counters_bytes, st));
+    if (int rc = plan_trace_long(ctx, b.max_len, b.cap_long)) return rc;
     if (timing) cudaEventRecord(ctx->ev[0], st);
     if (timing) cudaEventRecord(ctx->kev[0], st);
     for (int ti = 0; ti < n_t; ti++) {
@@ -848,9 +849,9 @@ static int run_sub(ab_context* ctx, Batch b, cudaStream_t st, bool timing, int s
     if (timing) cudaEventRecord(ctx->ev[1], st);
     k_scan_starts<<<sms * 8, 256, 0, st>>>(bv);
     if (timing) cudaEventRecord(ctx->kev[2], st);
-    k_trace<false><<<sms * ctx->grid_trace, 128, 0, st>>>(bv);
+    k_trace<false><<<sms * WALKER_CTAS_PER_SM, 128, 0, st>>>(bv);
     if (timing) cudaEventRecord(ctx->kev[3], st);
-    launch_trace_long(ctx, bv, st, sub);
+    launch_trace_long(ctx, bv, st);
     if (timing) cudaEventRecord(ctx->kev[4], st);
     k_emit<<<sms * 8, 128, 0, st>>>(bv);
     if (timing) cudaEventRecord(ctx->kev[5], st);
@@ -927,96 +928,9 @@ static int run_sub(ab_context* ctx, Batch b, cudaStream_t st, bool timing, int s
         CK(cudaGetLastError());
     }
     if (timing) cudaEventRecord(ctx->kev[12], st);
-    return AB_OK;
-}
-
-// board-stage buffers of this slot for the reserved geometry (maxB frames of capC markers)
-static int ensure_board_buffers(ab_context* ctx) {
-    if (ctx->board_frames >= ctx->maxB && ctx->board_capc == ctx->capC) return AB_OK;
-    auto F = [](auto*& p) {
-        if (p) cudaFree(p);
-        p = nullptr;
-    };
-    F(ctx->d_boards);
-    F(ctx->d_board_slots);
-    F(ctx->d_board_pts);
-    ctx->board_frames = ctx->board_capc = 0;
-    const size_t B = (size_t)ctx->maxB, C = (size_t)ctx->capC;
-    CK(cudaMalloc(&ctx->d_boards, B * sizeof(ab_board)));
-    CK(cudaMalloc(&ctx->d_board_slots, B * C * sizeof(int32_t)));
-    CK(cudaMalloc(&ctx->d_board_pts, B * C * BOARD_PTS_PER_MARKER * sizeof(float)));
-    ctx->board_frames = ctx->maxB;
-    ctx->board_capc = ctx->capC;
-    return AB_OK;
-}
-
-static int run_batch(ab_context* ctx, const uint8_t* dgrey, size_t row, size_t frame, int n, const float* K,
-                     const float* D, float marker_size) {
-    const ab_params& P = ctx->params;
-    if (P.decoder == AB_DECODER_HRM && !ctx->have_dict)
-        return set_err(ctx, AB_E_STATE, "HRM decoder selected but no dictionary loaded (ab_load_hrm_dictionary)");
-    if (P.decoder == AB_DECODER_HOST_CALLBACK && !ctx->cb)
-        return set_err(ctx, AB_E_STATE, "host-callback decoder selected but no callback set");
-    if (P.decoder == AB_DECODER_HRM && (ctx->dict.n + 2) > P.warp_size)
-        return set_err(ctx, AB_E_INVALID, "warp size too small for the dictionary");
-    if (P.corner_method == AB_CORNER_SUBPIX && ((int)P.thres_param1 < 1 || (int)P.thres_param1 > 24))
-        return set_err(ctx, AB_E_INVALID, "SUBPIX window %d outside 1..24", (int)P.thres_param1);
-    if (P.locked_corners && ((int)P.thres_param1 < 1 || (int)P.thres_param1 > 24))
-        return set_err(ctx, AB_E_INVALID, "locked-corner window %d outside 1..24", (int)P.thres_param1);
-    // setThresholdParamRange (markerdetector.h:152, cpp:322-334): 2*range+1 threshold images per frame, param1 =
-    // p1 - range + range*i (sic, SURVEY B.6); they live as n_t consecutive "virtual frames" per frame for the
-    // threshold / contour / polygon stages and are merged per frame by k_polygon's quad keys.
-    // CANNY ignores the parameters: the reference's 2r+1 identical edge images yield duplicate candidates that its
-    // too-near filter removes again (cpp:322-334, :592-627), so one image gives the same result.
-    const int n_t = n_thres_images(P);
-    if (n * n_t > ctx->maxB) return set_err(ctx, AB_E_STATE, "internal: %d virtual frames > reserved %d", n * n_t, ctx->maxB);
-    {   // k_scan_starts indexes its work items with 32 bits
-        const unsigned long long items = 8ull * (unsigned long long)((ctx->W + 31) >> 5) * (unsigned long long)((ctx->H + 2 + BIT_TILE - 1) / BIT_TILE) *
-                                         (unsigned long long)(n * n_t);
-        if (items >= (1ull << 32)) return set_err(ctx, AB_E_INVALID, "batch of %d frames %dx%d is too large for one launch: split it", n, ctx->W, ctx->H);
-    }
-    Batch b;
-    fill_batch(ctx, b, dgrey, row, frame, n, K, D, marker_size);
-    b.n_t = n_t;
-    if (ctx->have_board) {
-        if (int rc = ensure_board_buffers(ctx)) return rc;
-        b.boards = ctx->d_boards;
-        b.board_slots = ctx->d_board_slots;
-        b.board_pts = ctx->d_board_pts;
-    }
-    cudaStream_t st = ctx->stream;
-    CK(cudaMemsetAsync(ctx->d_counters, 0, ctx->counters_bytes, st));
-    // Sub-batch pipelining: several stages (long border walks, point emission, polygon fit, refinement, pose) are
-    // bound by dependent-load latency with few resident warps, others by instruction issue.  Two (or more) halves
-    // of the batch on separate streams let the latency-bound kernels of one half run under the issue-bound
-    // kernels of the other.  Every buffer is indexed by frame, so a sub-batch is just an offset view; the global
-    // append lists are partitioned by the per-frame capacities.  Per-kernel timing needs a single stream.
-    int nsub = 1;
-    if (!ctx->timing && P.decoder != AB_DECODER_HOST_CALLBACK && P.thres_method != AB_THRES_CANNY) {
-        nsub = ctx->n_sub_streams;
-        while (nsub > 1 && n < 8 * nsub) nsub--;
-    }
-    if (nsub > 1) {
-        CK(cudaEventRecord(ctx->ev_fork, st));
-        for (int s = 0; s < nsub; s++) CK(cudaStreamWaitEvent(ctx->sub_stream[s], ctx->ev_fork, 0));
-    }
-    if (int rc = plan_trace_long(ctx, b.max_len, ctx->capLongPF * (unsigned)(b.n_t * (n / nsub)), nsub)) return rc;
-    for (int s = 0; s < nsub; s++) {
-        const int f0 = (int)((long long)s * n / nsub), nf = (int)((long long)(s + 1) * n / nsub) - f0;
-        Batch v = sub_view(ctx, b, f0, nf, s);
-        int rc = run_sub(ctx, v, nsub > 1 ? ctx->sub_stream[s] : st, ctx->timing && nsub == 1, s);
-        if (rc) return rc;
-    }
-    if (nsub > 1) {
-        for (int s = 0; s < nsub; s++) {
-            CK(cudaEventRecord(ctx->ev_join[s], ctx->sub_stream[s]));
-            CK(cudaStreamWaitEvent(st, ctx->ev_join[s], 0));
-        }
-    }
     ctx->last = b;
     ctx->have_last = true;
     ctx->last_n = n;
-    ctx->last_nsub = nsub;
     return AB_OK;
 }
 
@@ -1051,7 +965,6 @@ static int get_twin(ab_context* ctx, ab_context** out) {
     t->cb = ctx->cb;
     t->cb_user = ctx->cb_user;
     t->timing = ctx->timing;
-    t->n_sub_streams = ctx->n_sub_streams;
     t->capLongPF = ctx->capLongPF;
     if (t->userQ != ctx->userQ || t->userC != ctx->userC || t->userStarts != ctx->userStarts || t->userPoints != ctx->userPoints) {
         free_buffers(t);
@@ -1142,11 +1055,9 @@ static int fetch_into(ab_context* ctx, ab_marker* out, int cap, int32_t* counts)
         }
     }
     CK(cudaStreamSynchronize(st));
-    Counters csum = *(const Counters*)ctx->h_counters;
-    for (int s2 = 1; s2 < MAX_SUB; s2++) csum.err |= ((const Counters*)ctx->h_counters)[s2].err;
-    int rc = check_device_errors(ctx, &csum);
+    int rc = check_device_errors(ctx, (const Counters*)ctx->h_counters);
     if (rc) return rc;
-    const unsigned* nm = (const unsigned*)(ctx->h_counters + MAX_SUB * sizeof(Counters)) + 2 * (size_t)ctx->maxB;
+    const unsigned* nm = (const unsigned*)(ctx->h_counters + FRAME_COUNTS_OFFSET) + 2 * (size_t)ctx->maxB;
     for (int f = 0; f < n; f++) {
         if ((int)nm[f] > cap && out)
             return set_err(ctx, AB_E_CAPACITY, "frame %d has %u markers but cap_per_frame is %d", f, nm[f], cap);
@@ -1385,18 +1296,13 @@ int ab_get_contour(ab_context* ctx, int frame, int candidate, int32_t* xy, int c
     CK(cudaStreamSynchronize(ctx->stream));
     CandRec cr;
     CK(cudaMemcpy(&cr, b.cands + (size_t)frame * b.cap_c + candidate, sizeof(CandRec), cudaMemcpyDeviceToHost));
-    // contour indices are relative to the list of the sub-batch that processed the frame
-    int sb = 0;
-    while (sb + 1 < ctx->last_nsub && frame >= (int)((long long)(sb + 1) * ctx->last_n / ctx->last_nsub)) sb++;
-    const int sf0 = (int)((long long)sb * ctx->last_n / ctx->last_nsub);
-    const ContourRec* cbase = b.contours + (size_t)ctx->capContoursPF * b.n_t * sf0;
-    const uint32_t* pbase = b.pool + (size_t)ctx->capPoolPF * b.n_t * sf0;
+    // contour indices and point offsets are relative to the start of the batch's lists
     ContourRec rec;
-    CK(cudaMemcpy(&rec, cbase + cr.contour, sizeof(ContourRec), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(&rec, b.contours + cr.contour, sizeof(ContourRec), cudaMemcpyDeviceToHost));
     *n = (int32_t)rec.n;
     if ((int)rec.n > cap_points) return set_err(ctx, AB_E_CAPACITY, "contour has %u points > cap %d", rec.n, cap_points);
     std::vector<uint32_t> p(rec.n);
-    CK(cudaMemcpy(p.data(), pbase + rec.off, sizeof(uint32_t) * rec.n, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(p.data(), b.pool + rec.off, sizeof(uint32_t) * rec.n, cudaMemcpyDeviceToHost));
     for (uint32_t i = 0; i < rec.n; i++) {
         uint32_t v = cr.swapped ? p[rec.n - 1 - i] : p[i];  // the reference reverses swapped contours (:622-625)
         xy[2 * i] = (int32_t)(v & 0xFFFFu);
@@ -1410,18 +1316,10 @@ int ab_get_counters(ab_context* ctx, int64_t* counters, int n) {
     if (!ctx || !ctx->have_last || !counters) return set_err(ctx, AB_E_INVALID, "no batch");
     cudaSetDevice(ctx->device);
     CK(cudaStreamSynchronize(ctx->stream));
-    Counters cs[MAX_SUB];
-    CK(cudaMemcpy(cs, ctx->d_counters, sizeof(cs), cudaMemcpyDeviceToHost));
-    int64_t v[6] = {0, 0, 0, 0, 0, 0};
-    for (int s2 = 0; s2 < MAX_SUB; s2++) {
-        const Counters& c = cs[s2];
-        v[0] += (int64_t)c.n_starts;
-        v[1] += (int64_t)c.n_contours;
-        v[2] += (int64_t)c.pool_used;
-        v[3] += (int64_t)c.n_quads_total;
-        v[4] += (int64_t)c.n_cands_total;
-        v[5] += (int64_t)c.n_markers_total;
-    }
+    Counters c;
+    CK(cudaMemcpy(&c, ctx->d_counters, sizeof(c), cudaMemcpyDeviceToHost));
+    const int64_t v[6] = {(int64_t)c.n_starts,      (int64_t)c.n_contours,    (int64_t)c.pool_used,
+                          (int64_t)c.n_quads_total, (int64_t)c.n_cands_total, (int64_t)c.n_markers_total};
     for (int i = 0; i < n && i < 6; i++) counters[i] = v[i];
     return AB_OK;
 }
@@ -1460,7 +1358,7 @@ int ab_threshold(ab_context* ctx, const uint8_t* grey, int width, int height, si
     if (param2 == -1) param2 = ctx->params.thres_param2;
     CK(cudaMemcpy2DAsync(ctx->d_grey[0], width, grey, row_stride, width, height, cudaMemcpyHostToDevice, ctx->stream));
     Batch b;
-    fill_batch(ctx, b, ctx->d_grey[0], width, (size_t)width * height, 1, nullptr, nullptr, -1.f);
+    fill_batch(ctx, b, ctx->d_grey[0], width, (size_t)width * height, 1, 1, nullptr, nullptr, -1.f);
     ctx->worker_call = true;
     rc = launch_threshold(ctx, b, method, param1, param2);
     ctx->worker_call = false;
@@ -1483,15 +1381,15 @@ int ab_detect_rectangles(ab_context* ctx, const uint8_t* thres, int width, int h
     cudaStream_t st = ctx->stream;
     CK(cudaMemcpy2DAsync(ctx->d_grey[0], width, thres, row_stride, width, height, cudaMemcpyHostToDevice, st));
     Batch b;
-    fill_batch(ctx, b, ctx->d_grey[0], width, (size_t)width * height, 1, nullptr, nullptr, -1.f);
+    fill_batch(ctx, b, ctx->d_grey[0], width, (size_t)width * height, 1, 1, nullptr, nullptr, -1.f);
     CK(cudaMemsetAsync(ctx->d_counters, 0, ctx->counters_bytes, st));
     k_threshold_fixed<<<ctx->sm_count * 8, 256, 0, st>>>(b.grey, b.grey_row, b.grey_frame, b.thres, b.bits, b.bits_words, b.W, b.H,
                                                           b.wpr, 0, 1, 1, 1, 0);
     k_scan_starts<<<ctx->sm_count * 8, 256, 0, st>>>(b);
-    k_trace<false><<<ctx->sm_count * 8, 128, 0, st>>>(b);
-    rc = plan_trace_long(ctx, b.max_len, b.cap_long, 1);
+    k_trace<false><<<ctx->sm_count * WALKER_CTAS_PER_SM, 128, 0, st>>>(b);
+    rc = plan_trace_long(ctx, b.max_len, b.cap_long);
     if (rc) return rc;
-    launch_trace_long(ctx, b, st, 0);
+    launch_trace_long(ctx, b, st);
     k_emit<<<ctx->sm_count * 8, 128, 0, st>>>(b);
     k_polygon<<<ctx->sm_count * 4, 128, 0, st>>>(b);
     k_frame_filter<<<1, 256, 0, st>>>(b);
@@ -1499,7 +1397,6 @@ int ab_detect_rectangles(ab_context* ctx, const uint8_t* thres, int width, int h
     ctx->last = b;
     ctx->have_last = true;
     ctx->last_n = 1;
-    ctx->last_nsub = 1;
     CK(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, ctx->counters_bytes, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     rc = check_device_errors(ctx, (const Counters*)ctx->h_counters);

@@ -121,23 +121,12 @@ __global__ void __launch_bounds__(256) k_scan_starts(Batch b) {
 // (full walker state) and its lane is refilled; k_trace<true> then runs the parked walks to completion in
 // densely populated warps.  Without this, the long walks end up one or two per warp and the kernel spends
 // most of its time issuing instructions for ~9 of 32 lanes (ncu r1e).
-#ifndef AB_TRACE_LONG_T
-#define AB_TRACE_LONG_T 48
-#endif
-#ifndef AB_TRACE_STEPS
-#define AB_TRACE_STEPS 8
-#endif
-#ifndef AB_TRACE_STEPS_LONG
-#define AB_TRACE_STEPS_LONG 8
-#endif
-#ifndef AB_EMIT_STEPS
-#define AB_EMIT_STEPS 16
-#endif
-constexpr int TRACE_LONG_T = AB_TRACE_LONG_T;
-// iterations a walk has made when k_trace<false> parks it: lanes are refilled only between rounds of AB_TRACE_STEPS
+constexpr int TRACE_LONG_T = 48;
+constexpr int TRACE_STEPS = 8, TRACE_STEPS_LONG = 8;  // iterations per round of k_trace<false> / k_trace<true>
+// iterations a walk has made when k_trace<false> parks it: lanes are refilled only between rounds of TRACE_STEPS
 // iterations, so the count is the first multiple of the round length that reaches the parking threshold
-constexpr int TRACE_PARK_N = (AB_TRACE_LONG_T + AB_TRACE_STEPS - 1) / AB_TRACE_STEPS * AB_TRACE_STEPS;
-static_assert(TRACE_PARK_N % 2 == 0 && AB_TRACE_STEPS_LONG % 2 == 0, "paired strip stores need even rounds");
+constexpr int TRACE_PARK_N = (TRACE_LONG_T + TRACE_STEPS - 1) / TRACE_STEPS * TRACE_STEPS;
+static_assert(TRACE_PARK_N % 2 == 0 && TRACE_STEPS_LONG % 2 == 0, "paired strip stores need even rounds");
 
 // `s` is the start state of a start candidate (table flags e): does its trigger scan before key0?
 // (raster positions fit 32 bits: W, H <= 16384)
@@ -148,7 +137,7 @@ __device__ __forceinline__ bool smaller_trigger(uint32_t e, const WalkState& s, 
 
 template <bool LONG>
 __global__ void __launch_bounds__(128) k_trace(Batch b) {
-    constexpr int STEPS = LONG ? AB_TRACE_STEPS_LONG : AB_TRACE_STEPS;
+    constexpr int STEPS = LONG ? TRACE_STEPS_LONG : TRACE_STEPS;
     const unsigned FULL = 0xFFFFFFFFu;
     const int lane = threadIdx.x & 31;
     unsigned long long n_items;
@@ -165,18 +154,8 @@ __global__ void __launch_bounds__(128) k_trace(Batch b) {
     TraceStart st{0, 0, 0, 0};
     WalkState fw{0, 0, 0}, bw{0, 0, 0};
     uint32_t e_fw = 0, type_bit = 0;  // e_fw: forward table entry of the current forward state
-#ifdef AB_TRACE_SMEM_LUT
-    // variant study: the two 4 KB step tables in shared memory instead of L1-cached global memory
-    __shared__ __align__(16) uint8_t s_lut[2 * WALK_LUT_SIZE];
-    for (int i = threadIdx.x; i < 2 * WALK_LUT_SIZE / 16; i += blockDim.x)
-        reinterpret_cast<uint4*>(s_lut)[i] = reinterpret_cast<const uint4*>(b.walk_lut)[i];
-    __syncthreads();
-    const uint8_t* lut_fw = s_lut;
-    const uint8_t* lut_bw = s_lut + WALK_LUT_SIZE;
-#else
     const uint8_t* __restrict__ lut_fw = b.walk_lut;
     const uint8_t* __restrict__ lut_bw = b.walk_lut + WALK_LUT_SIZE;
-#endif
     int nf = 0, ng = 0, frame = 0;
     // LONG only: entry k of the lane's strip = (pixel of the forward walker after TRACE_PARK_N + 1 + k steps, pixel of the
     // backward walker after as many) = points TRACE_PARK_N + 1 + k and n - TRACE_PARK_N - 1 - k of the contour.  Losers

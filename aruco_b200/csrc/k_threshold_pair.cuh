@@ -17,18 +17,9 @@
 #pragma once
 #include "k_threshold_fast.cuh"
 
-// tuning knobs (variant studies build with -D...)
-#ifndef AB_THP_RH
-#define AB_THP_RH 128
-#endif
-#ifndef AB_THP_DEPTH
-#define AB_THP_DEPTH 8
-#endif
-#ifndef AB_THP_MINB
-#define AB_THP_MINB 1
-#endif
-
 namespace ab {
+
+constexpr int THP_RH = 128;  // output rows per CTA before rounding down to whole double turns of the ring
 
 template <uint32_t SEL>
 __device__ __forceinline__ uint32_t prmt(uint32_t a, uint32_t b) {
@@ -52,13 +43,13 @@ __device__ __forceinline__ void lds128(uint32_t addr, uint32_t& x, uint32_t& y, 
 // Requires W % 4 == 0 and 4-byte aligned source rows (the dispatcher checks): a thread's 4 columns are then either all
 // inside the image, all left of it or all right of it, and the replicated border is a PRMT selector, not a branch.
 template <int K, int TO>
-__global__ void __launch_bounds__(TO + 32, AB_THP_MINB) k_threshold_pair(ThrArgs a) {
+__global__ void __launch_bounds__(TO + 32, 1) k_threshold_pair(ThrArgs a) {
     constexpr int R = K / 2, R4 = (R + 3) & ~3, HT = R4 / 4, NV = 4 + 2 * R4, HO = 4 * TO, TW = 2 * HO, CSW = HO + 2 * R4, K2 = K * K;
     constexpr uint32_t BUF_BYTES = CSW * 4;
     constexpr int NT = TO + 2 * HT;              // working threads
-    constexpr int DEPTH = AB_THP_DEPTH;                     // source rows in flight (cp.async groups)
+    constexpr int DEPTH = 8;                     // source rows in flight (cp.async groups)
     constexpr uint32_t STAGE_ROW = NT * 8;       // bytes of one staged row: 2 words per thread
-    constexpr int RH = (AB_THP_RH / (2 * K)) * (2 * K);  // rows per CTA: whole double turns of the ring, so the unrolled loop has no exits
+    constexpr int RH = (THP_RH / (2 * K)) * (2 * K);  // rows per CTA: whole double turns of the ring, so the unrolled loop has no exits
     __shared__ __align__(16) uint32_t cs[4][CSW];  // two buffers of two rows
     __shared__ __align__(16) uint2 stage[DEPTH][NT];  // ncu r1j: with loads held in registers two of the K unrolled steps
                                                       // waited ~1 row on the scoreboard; cp.async groups decouple them
@@ -208,7 +199,7 @@ inline bool launch_threshold_pair(const ThrArgs& a, int B, cudaStream_t st) {
         if (pad < best_pad) best_pad = pad, best_to = to;
     }
     const int tw = 8 * best_to;
-    const int rh = (AB_THP_RH / (2 * a.k)) * (2 * a.k);
+    const int rh = (THP_RH / (2 * a.k)) * (2 * a.k);
     dim3 grid((a.W + tw - 1) / tw, (a.H + rh - 1) / rh, B);
 #define AB_THP_TO(KK, TT)                                        \
     if (best_to == TT) {                                         \

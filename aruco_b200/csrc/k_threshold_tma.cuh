@@ -13,53 +13,25 @@
 //     the row predicate exists only in the instantiation used for the last, partial row group of the bottom CTA row,
 //   * a thread reads its two source words with immediate-offset shared loads (row slots are compile-time inside the
 //     unrolled 2K-row body).
-// Shared memory per CTA: (NG x 2K + 2R) staged rows of TW + 32 bytes (pitch rounded up to 128) + the 4 column-sum rows:
-// 49 KB for K = 7, TO = 96.
+// Shared memory per CTA: NG x 2K staged rows of TW + 32 bytes (pitch rounded up to 128) + the 4 column-sum rows:
+// 31.4 KB for K = 7, TO = 96.
 #pragma once
 #include <cuda.h>
 #include "k_threshold_pair.cuh"
 
-#ifndef AB_THT_NG
-#define AB_THT_NG 2  // row groups in flight (r2c: 2 -> 1.33 ms, 3 -> 1.34 ms, 4 -> 1.57 ms; shared memory taken here is L1 taken from co-running kernels)
-#endif
-#ifndef AB_THT_RH
-#define AB_THT_RH 128
-#endif
-#ifndef AB_THT_MINB
-#define AB_THT_MINB 1
-#endif
-#ifndef AB_THT_RPB
-#define AB_THT_RPB 2  // rows per CTA barrier: 2, or 0 = K (half a group)
-#endif
-#ifndef AB_THT_OWN
-#define AB_THT_OWN 1  // a thread's own column sums stay in registers (two 16-byte shared loads per row instead of three)
-#endif
-#ifndef AB_THT_PREF_TO
-#define AB_THT_PREF_TO 96
-#endif
-#ifndef AB_THT_PRIME_IN_SLOT
-#define AB_THT_PRIME_IN_SLOT 1  // 1: the 2R priming rows borrow the last group slot (its group is issued after they are consumed)
-#endif
-#ifndef AB_THW_GR
-#define AB_THW_GR 8  // wide kernel: rows per TMA group (r2q, K = 21: 8 -> 0.56 ms, 10 -> 0.61, 14 -> 0.62 per 64 frames; 43 instead of 54 KB per CTA)
-#endif
-#ifndef AB_THT_SHFL
-#define AB_THT_SHFL 0  // 1: the neighbours' column sums come by warp shuffle; shared memory only carries them across warp edges
-#endif
-#ifndef AB_THT_PIPE
-#define AB_THT_PIPE 0  // 1: split arrive / wait (finish the rows of pair p while the barrier of pair p+1 fills): correct, no gain (r2k: 1.276 vs 1.282 ms)
-#endif
-
 namespace ab {
+
+// row groups in flight (r2c: 2 -> 1.33 ms, 3 -> 1.34 ms, 4 -> 1.57 ms; shared memory taken here is L1 taken from co-running kernels)
+constexpr int THT_NG = 2;
+constexpr int THT_RH = 128;  // output rows per CTA before rounding down to whole groups
+// wide kernel: rows per TMA group (r2q, K = 21: 8 -> 0.56 ms, 10 -> 0.61, 14 -> 0.62 per 64 frames; 43 instead of 54 KB per CTA)
+constexpr int THW_GR = 8;
 
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
 }
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     asm volatile(
@@ -91,35 +63,26 @@ struct ThrTmaArgs {
 };
 
 template <int K, int TO, bool U8>
-__global__ void __launch_bounds__(TO + 32, AB_THT_MINB) k_threshold_tma(const __grid_constant__ CUtensorMap src_map, ThrTmaArgs a) {
+__global__ void __launch_bounds__(TO + 32, 1) k_threshold_tma(const __grid_constant__ CUtensorMap src_map, ThrTmaArgs a) {
     constexpr int R = K / 2, R4 = (R + 3) & ~3, HT = R4 / 4, NV = 4 + 2 * R4, HO = 4 * TO, TW = 2 * HO, CSW = HO + 2 * R4, K2 = K * K;
     constexpr uint32_t BUF_BYTES = CSW * 4;
     constexpr int NT = TO + 2 * HT;            // working threads
     constexpr int GR = 2 * K;                  // rows per group = one unrolled body
-    constexpr int NG = AB_THT_NG;              // groups in flight
+    constexpr int NG = THT_NG;                 // groups in flight
     constexpr int ROWB = TW + 32;              // staged bytes per row: columns X0-16 .. X0+TW+15 (TMA: 16-byte aligned start)
     constexpr int ROWP = (ROWB + 127) & ~127;  // row pitch in shared memory: TMA destinations are 128-byte aligned
-    constexpr int RH = (AB_THT_RH / GR) * GR;  // output rows per CTA
-    constexpr int RPB = AB_THT_RPB ? AB_THT_RPB : K;  // rows published per CTA barrier
-    constexpr bool OWN = AB_THT_OWN && RPB == 2 && R4 == 4;
-    // PIPE: ncu r2i -- the CTA barrier between publishing the column sums of a row pair and reading the neighbours' was the
-    // top stall (2.7 of 7.8 cycles per issued instruction).  An mbarrier splits it: a thread ARRIVES after publishing row
-    // pair p+1, then finishes the output rows of pair p (whose sums became visible at the previous wait), and only then
-    // WAITS for pair p+1.  Three column-sum buffers, because a fast thread publishes pair p+2 while a slow one still reads
-    // pair p.  The centre-row ring slots of pair p survive the two ring steps of pair p+1 for K >= 7.
-    constexpr bool SHFL = AB_THT_SHFL && OWN && !AB_THT_PIPE;
-    constexpr bool PIPE = AB_THT_PIPE && RPB == 2 && K >= 7;
-    constexpr int NBUF = PIPE ? 3 : 2;
-    static_assert(GR % RPB == 0, "rows per barrier must divide the group");
+    constexpr int RH = (THT_RH / GR) * GR;     // output rows per CTA
+    constexpr bool OWN = R4 == 4;  // a thread's own column sums stay in registers (two 16-byte shared loads per row instead of three)
+    static_assert(NG >= 2 && 2 * R <= GR, "the priming rows borrow the last group slot");
     static_assert(ROWB % 16 == 0 && R4 <= 8, "TMA box: inner extent must be a multiple of 16 bytes");
-    // dynamic shared memory: staged rows (groups, then the 2R priming rows) | 4 column-sum rows (two buffers of two) | barriers
+    // dynamic shared memory: staged rows (NG groups) | 4 column-sum rows (two buffers of two) | barriers (NG groups, priming).
+    // The 2R priming rows borrow the last group slot; its group is issued after they are consumed.
     extern __shared__ __align__(128) uint8_t tht_smem[];
-    constexpr bool PSLOT = AB_THT_PRIME_IN_SLOT && NG >= 2 && 2 * R <= GR;
-    constexpr int PRIME_ROW0 = PSLOT ? (NG - 1) * GR : NG * GR;
-    constexpr int STAGE_BYTES = (PSLOT ? NG * GR : NG * GR + 2 * R) * ROWP;
+    constexpr int PRIME_ROW0 = (NG - 1) * GR;
+    constexpr int STAGE_BYTES = NG * GR * ROWP;
     uint8_t* stage = tht_smem;
     uint32_t* cs = reinterpret_cast<uint32_t*>(tht_smem + STAGE_BYTES);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(tht_smem + STAGE_BYTES + NBUF * RPB * BUF_BYTES);  // NG groups, priming, phases
+    uint64_t* bars = reinterpret_cast<uint64_t*>(tht_smem + STAGE_BYTES + 4 * BUF_BYTES);
     const int t = threadIdx.x;
     const int X0 = blockIdx.x * TW, y0 = blockIdx.y * RH, f = blockIdx.z;
     const int nout = min(RH, a.H - y0);
@@ -138,14 +101,13 @@ __global__ void __launch_bounds__(TO + 32, AB_THT_MINB) k_threshold_tma(const __
     if (t == 0) {
 #pragma unroll
         for (int i = 0; i <= NG; i++) mbar_init(s_bars + 8u * i, 1);
-        mbar_init(s_bars + 8u * (NG + 1), NT);  // PIPE: every working thread arrives once per row pair
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         // priming rows y0-R .. y0+R-1, then the first groups
         const uint32_t pbar = s_bars + 8u * NG;
         mbar_expect_tx(pbar, 2 * R * ROWB);
         for (int r = 0; r < 2 * R; r++)
             tma_load_row(s_stage + (uint32_t)((PRIME_ROW0 + r) * ROWP), &src_map, (X0 - 16) >> 2, min(max(y0 - R + r, 0), a.H - 1), f, pbar);
-        for (int g = 0; g < (PSLOT ? NG - 1 : NG) && g < ngroups; g++) issue_group(g);
+        for (int g = 0; g < NG - 1 && g < ngroups; g++) issue_group(g);
     }
     __syncthreads();  // barrier words initialised before anybody polls them
     const bool is_out = t < TO;
@@ -178,11 +140,6 @@ __global__ void __launch_bounds__(TO + 32, AB_THT_MINB) k_threshold_tma(const __
     const uint32_t s_wr = s_base + 4u * ci, s_rd = s_base + 4u * (ci - R4);
     const int nib_shift = 4 * (t & 3);
     uint32_t boff = 0;
-    // SHFL: who publishes its sums to shared memory (the lanes at warp edges and the halo threads) and who reads a
-    // neighbour's from there (the others get them by shuffle)
-    const int lane_id = t & 31;
-    const bool pub = lane_id == 0 || lane_id == 31 || !is_out || t == TO - 1;
-    const bool need_l = lane_id == 0, need_r = lane_id == 31 || t == TO - 1;
 
     uint32_t ring[K][4];
     uint32_t V0 = 0u, V1 = 0u, V2 = 0u, V3 = 0u;
@@ -209,46 +166,16 @@ __global__ void __launch_bounds__(TO + 32, AB_THT_MINB) k_threshold_tma(const __
     mbar_wait(s_bars + 8u * NG, 0);
 #pragma unroll
     for (int j = 0; j < 2 * R; j++) accumulate(s_stage + (uint32_t)((PRIME_ROW0 + j) * ROWP), ring[j], true);
-    if (PSLOT) {  // the borrowed slot is free again
-        __syncthreads();
-        if (t == 0 && NG - 1 < ngroups) issue_group(NG - 1);
-    }
+    __syncthreads();  // the borrowed slot is free again
+    if (t == 0 && NG - 1 < ngroups) issue_group(NG - 1);
 #pragma unroll
     for (int j = 2 * R; j < K; j++) ring[j][0] = ring[j][1] = ring[j][2] = ring[j][3] = 0u;
     // horizontal window sums, comparison and stores of one output row whose column sums sit at shared offset `rd`
     auto emit_row = [&](uint32_t rd, const uint32_t* c, bool row_ok, const uint32_t* own) {
         uint32_t w[NV];
-        if (SHFL) {
-            w[4] = own[0], w[5] = own[1], w[6] = own[2], w[7] = own[3];
-            w[0] = 0u;
-            w[11] = 0u;
-#pragma unroll
-            for (int q = 1; q < 4; q++) w[q] = __shfl_up_sync(out_mask, own[q], 1);        // left neighbour's sums 1..3
-#pragma unroll
-            for (int q = 0; q < 3; q++) w[8 + q] = __shfl_down_sync(out_mask, own[q], 1);  // right neighbour's sums 0..2
-            if (R == 4) {
-                w[0] = __shfl_up_sync(out_mask, own[0], 1);
-                w[11] = __shfl_down_sync(out_mask, own[3], 1);
-            }
-            if (need_l) lds128(rd, w[0], w[1], w[2], w[3]);
-            if (need_r) lds128(rd + 32u, w[8], w[9], w[10], w[11]);
-        } else if (OWN) {  // the middle four entries are this thread's own sums
-#if defined(AB_THT_MINLDS)
-            // variant study: only the six neighbour entries a 7-wide window needs (two 8-byte + two 4-byte loads: 6 wavefronts
-            // per warp instead of 8)
-            if (R <= 3) {
-                w[0] = 0u;
-                w[11] = 0u;
-                asm volatile("ld.shared.b32 %0, [%1];" : "=r"(w[1]) : "r"(rd + 4u) : "memory");
-                asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(w[2]), "=r"(w[3]) : "r"(rd + 8u) : "memory");
-                asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(w[8]), "=r"(w[9]) : "r"(rd + 32u) : "memory");
-                asm volatile("ld.shared.b32 %0, [%1];" : "=r"(w[10]) : "r"(rd + 40u) : "memory");
-            } else
-#endif
-            {
-                lds128(rd, w[0], w[1], w[2], w[3]);
-                lds128(rd + 32u, w[8], w[9], w[10], w[11]);
-            }
+        if (OWN) {  // the middle four entries are this thread's own sums
+            lds128(rd, w[0], w[1], w[2], w[3]);
+            lds128(rd + 32u, w[8], w[9], w[10], w[11]);
             w[4] = own[0], w[5] = own[1], w[6] = own[2], w[7] = own[3];
         } else {
 #pragma unroll
@@ -288,73 +215,32 @@ __global__ void __launch_bounds__(TO + 32, AB_THT_MINB) k_threshold_tma(const __
     auto body = [&](uint32_t gbase, int o, auto tail) {
         constexpr bool TAIL = decltype(tail)::value;
 #pragma unroll
-        for (int jj = 0; jj < GR; jj += RPB) {
+        for (int jj = 0; jj < GR; jj += 2) {
             uint32_t own[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
-            for (int q = 0; q < RPB; q++) {
+            for (int q = 0; q < 2; q++) {
                 accumulate(gbase + (uint32_t)((jj + q) * ROWP), ring[(2 * R + jj + q) % K], false);
-                if (!SHFL || pub) sts128(s_wr + boff + q * BUF_BYTES, V0, V1, V2, V3);
+                sts128(s_wr + boff + q * BUF_BYTES, V0, V1, V2, V3);
                 if (OWN && q == 0) own[0] = V0, own[1] = V1, own[2] = V2, own[3] = V3;
             }
             __syncthreads();
             if (is_out) {
                 const uint32_t cur[4] = {V0, V1, V2, V3};
 #pragma unroll
-                for (int q = 0; q < RPB; q++)
+                for (int q = 0; q < 2; q++)
                     emit_row(s_rd + boff + q * BUF_BYTES, ring[(R + jj + q) % K], !TAIL || o + jj + q < nout, q == 0 ? own : cur);
             }
-            boff = RPB * BUF_BYTES - boff;
+            boff = 2 * BUF_BYTES - boff;
         }
     };
-    if (!PIPE) {
-        for (int g = 0; g < ngroups; g++) {
-            const int slot = g % NG;
-            mbar_wait(s_bars + 8u * (uint32_t)slot, (uint32_t)((g / NG) & 1));
-            const uint32_t gbase = s_stage + (uint32_t)(slot * GR * ROWP);
-            if ((g + 1) * GR <= nout) body(gbase, g * GR, std::false_type{});
-            else body(gbase, g * GR, std::true_type{});
-            // every thread is past its last read of this slot (the body ends behind a CTA barrier): refill it
-            if (t == 0 && g + NG < ngroups) issue_group(g + NG);
-        }
-    } else {
-        const uint32_t phbar = s_bars + 8u * (NG + 1);
-        uint32_t wr = 0, rd = 0, parity = 0;  // column-sum buffer written by the current pair / read for the previous pair
-        uint32_t oa[4] = {0u, 0u, 0u, 0u}, ob[4] = {0u, 0u, 0u, 0u};  // own sums of the pair that is finished next
-        int orow_i = 0;                                                // first output row of that pair
-        for (int g = 0; g < ngroups; g++) {
-            const int slot = g % NG;
-            mbar_wait(s_bars + 8u * (uint32_t)slot, (uint32_t)((g / NG) & 1));
-            const uint32_t gbase = s_stage + (uint32_t)(slot * GR * ROWP);
-#pragma unroll
-            for (int jj = 0; jj < GR; jj += 2) {
-                accumulate(gbase + (uint32_t)(jj * ROWP), ring[(2 * R + jj) % K], false);
-                sts128(s_wr + wr, V0, V1, V2, V3);
-                const uint32_t na[4] = {V0, V1, V2, V3};
-                accumulate(gbase + (uint32_t)((jj + 1) * ROWP), ring[(2 * R + jj + 1) % K], false);
-                sts128(s_wr + wr + BUF_BYTES, V0, V1, V2, V3);
-                const uint32_t nb[4] = {V0, V1, V2, V3};
-                mbar_arrive(phbar);
-                if (is_out && (jj > 0 || g > 0)) {  // the previous pair: its sums became visible at the last wait
-                    const int pj = (jj + GR - 2) % GR;
-                    emit_row(s_rd + rd, ring[(R + pj) % K], orow_i < nout, oa);
-                    emit_row(s_rd + rd + BUF_BYTES, ring[(R + pj + 1) % K], orow_i + 1 < nout, ob);
-                    orow_i += 2;
-                }
-                mbar_wait(phbar, parity);
-                parity ^= 1u;
-                rd = wr;
-                wr = wr == 2 * 2 * BUF_BYTES ? 0u : wr + 2 * BUF_BYTES;
-#pragma unroll
-                for (int q = 0; q < 4; q++) oa[q] = na[q], ob[q] = nb[q];
-            }
-            // every thread has passed the wait behind its last read of this slot: refill it
-            if (t == 0 && g + NG < ngroups) issue_group(g + NG);
-        }
-        if (is_out) {  // the last pair
-            constexpr int pj = GR - 2;
-            emit_row(s_rd + rd, ring[(R + pj) % K], orow_i < nout, oa);
-            emit_row(s_rd + rd + BUF_BYTES, ring[(R + pj + 1) % K], orow_i + 1 < nout, ob);
-        }
+    for (int g = 0; g < ngroups; g++) {
+        const int slot = g % NG;
+        mbar_wait(s_bars + 8u * (uint32_t)slot, (uint32_t)((g / NG) & 1));
+        const uint32_t gbase = s_stage + (uint32_t)(slot * GR * ROWP);
+        if ((g + 1) * GR <= nout) body(gbase, g * GR, std::false_type{});
+        else body(gbase, g * GR, std::true_type{});
+        // every thread is past its last read of this slot (the body ends behind a CTA barrier): refill it
+        if (t == 0 && g + NG < ngroups) issue_group(g + NG);
     }
 }
 
@@ -372,10 +258,10 @@ __global__ void __launch_bounds__(TO + 32, 1) k_threshold_tma_wide(const __grid_
     constexpr int R = K / 2, R4 = (R + 3) & ~3, HT = R4 / 4, NV = 4 + 2 * R4, HO = 4 * TO, TW = 2 * HO, CSW = HO + 2 * R4, K2 = K * K;
     constexpr uint32_t BUF_BYTES = CSW * 4;
     constexpr int NT = TO + 2 * HT;
-    constexpr int GR = AB_THW_GR;              // rows per TMA group = one unrolled body
+    constexpr int GR = THW_GR;                 // rows per TMA group = one unrolled body
     constexpr int NS = K + 2 * GR + 3;         // staged rows (ring); row NS is a row of zeros
     constexpr int ROWB = TW + 32, ROWP = (ROWB + 127) & ~127;
-    constexpr int RH = (AB_THT_RH / GR) * GR;
+    constexpr int RH = (THT_RH / GR) * GR;
     constexpr int CH = 65535 / (255 * K);      // packed terms that cannot overflow a 16-bit lane
     static_assert(R4 <= 16, "halo of the staged tile is 16 columns");
     extern __shared__ __align__(128) uint8_t tht_smem[];
@@ -551,7 +437,6 @@ inline ab_encode_tiled_fn tensor_map_encoder() {
 
 // the TO whose tile width 8*TO divides W (widest first); 0 if none
 inline int threshold_tma_tile(int W) {
-    if (W % (8 * AB_THT_PREF_TO) == 0) return AB_THT_PREF_TO;
     for (int to : {96, 120, 80, 64, 40})  // (8 TO + 32) / 4 <= 256: the TMA box limit
         if (W % (8 * to) == 0) return to;
     return 0;
@@ -559,14 +444,11 @@ inline int threshold_tma_tile(int W) {
 
 constexpr size_t threshold_tma_wide_smem(int K, int TO) {
     const int R = K / 2, R4 = (R + 3) & ~3, HO = 4 * TO, TW = 2 * HO, CSW = HO + 2 * R4;
-    return (size_t)(K + 2 * AB_THW_GR + 4) * (size_t)((TW + 32 + 127) & ~127) + 4 * (size_t)CSW * 4 + 8 * 4;
+    return (size_t)(K + 2 * THW_GR + 4) * (size_t)((TW + 32 + 127) & ~127) + 4 * (size_t)CSW * 4 + 8 * 4;
 }
 constexpr size_t threshold_tma_smem(int K, int TO) {
     const int R = K / 2, R4 = (R + 3) & ~3, HO = 4 * TO, TW = 2 * HO, CSW = HO + 2 * R4;
-    const int RPB = AB_THT_RPB ? AB_THT_RPB : K;
-    const int NBUF = (AB_THT_PIPE && RPB == 2 && K >= 7) ? 3 : 2;
-    const bool PSLOT = AB_THT_PRIME_IN_SLOT && AB_THT_NG >= 2;  // 2R <= 2K always
-    return (size_t)(AB_THT_NG * 2 * K + (PSLOT ? 0 : 2 * R)) * (size_t)((TW + 32 + 127) & ~127) + NBUF * RPB * (size_t)CSW * 4 + 8 * (AB_THT_NG + 2);
+    return (size_t)(THT_NG * 2 * K) * (size_t)((TW + 32 + 127) & ~127) + 4 * (size_t)CSW * 4 + 8 * (THT_NG + 1);
 }
 template <class KERNEL>
 inline void threshold_tma_launch(KERNEL kern, dim3 grid, int threads, size_t smem, cudaStream_t st, const CUtensorMap& map, const ThrTmaArgs& ta) {
@@ -587,17 +469,11 @@ inline void threshold_tma_launch(KERNEL kern, dim3 grid, int threads, size_t sme
 
 // returns false when the TMA path does not apply (alignment, tile divisibility, lane budget): the caller falls back
 inline bool launch_threshold_tma(const ThrArgs& a, int B, cudaStream_t st) {
-    static const bool disabled = getenv("ARUCO_B200_NO_TMA") != nullptr;
-    if (disabled) return false;
     const int K2 = a.k * a.k;
     const long long cst = (long long)K2 * a.idelta - (K2 - 1) / 2;
     if (a.k < 3 || a.k > 21 || !(a.k & 1) || (a.W & 3)) return false;
-#ifdef AB_THT_FORCE_WIDE7
-    const bool wide = a.k >= 13 || a.k == 7;  // variant study: the ring-less kernel for the default block size
-#else
     const bool wide = a.k >= 13 || K2 * 255LL + (cst < 0 ? -cst : cst) >= 0x8000;  // the window sums leave the 16-bit lanes
     if (wide && a.k < 13) return false;
-#endif
     if ((((uintptr_t)a.grey) | a.grey_row | a.grey_frame) & 15) return false;  // TMA: 16-byte aligned base and strides
     const int to = threshold_tma_tile(a.W);
     ab_encode_tiled_fn enc = tensor_map_encoder();
@@ -611,7 +487,7 @@ inline bool launch_threshold_tma(const ThrArgs& a, int B, cudaStream_t st) {
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
         return false;
     ThrTmaArgs ta{a.thres, a.bits, a.bits_words, a.W, a.H, a.wpr, a.idelta, a.out_mul, a.out_off};
-    const int rh = wide ? (AB_THT_RH / AB_THW_GR) * AB_THW_GR : (AB_THT_RH / (2 * a.k)) * (2 * a.k);
+    const int rh = wide ? (THT_RH / THW_GR) * THW_GR : (THT_RH / (2 * a.k)) * (2 * a.k);
     dim3 grid(a.W / tw, (a.H + rh - 1) / rh, B);
     if (wide) {
 #define AB_THW_TO(KK, TT)                                                                                                \
@@ -625,9 +501,6 @@ inline bool launch_threshold_tma(const ThrArgs& a, int B, cudaStream_t st) {
     case KK:            \
         AB_THW_TO(KK, 96) AB_THW_TO(KK, 120) AB_THW_TO(KK, 80) AB_THW_TO(KK, 40) return false;
         switch (a.k) {
-#ifdef AB_THT_FORCE_WIDE7
-            AB_THW_CASE(7)
-#endif
             AB_THW_CASE(13)
             AB_THW_CASE(15)
             AB_THW_CASE(17)
