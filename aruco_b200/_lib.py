@@ -62,6 +62,7 @@ SYMBOLS = {
     "ab_get_grey": (_i, [_vp, _i, _vp, _sz]),
     "ab_get_candidates": (_i, [_vp, _i, _vp, _vp, _vp, _i, C.POINTER(C.c_int32)]),
     "ab_get_canonical": (_i, [_vp, _i, _i, _vp]),
+    "ab_get_canonical_size": (_i, [_vp, C.POINTER(C.c_int32)]),
     "ab_get_contour": (_i, [_vp, _i, _i, _vp, _i, C.POINTER(C.c_int32)]),
     "ab_get_counters": (_i, [_vp, _vp, _i]),
     "ab_enable_timing": (_i, [_vp, _i]),

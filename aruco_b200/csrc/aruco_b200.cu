@@ -1287,6 +1287,13 @@ int ab_get_canonical(ab_context* ctx, int frame, int candidate, uint8_t* dst) {
     return AB_OK;
 }
 
+int ab_get_canonical_size(ab_context* ctx, int32_t* size) {
+    if (ctx) ctx = current_of(ctx);
+    if (!ctx || !ctx->have_last || !size) return set_err(ctx, AB_E_STATE, "no batch");
+    *size = ctx->last.S;
+    return AB_OK;
+}
+
 int ab_get_contour(ab_context* ctx, int frame, int candidate, int32_t* xy, int cap_points, int32_t* n) {
     if (ctx) ctx = current_of(ctx);
     if (!ctx || !ctx->have_last || frame < 0 || frame >= ctx->last_n || !n || candidate < 0 || candidate >= ctx->last.cap_c)

@@ -91,8 +91,8 @@ __global__ void __launch_bounds__(64) k_homography(Batch b) {
 //    host-callback decoders and k_identify read it) and its 256-bin histogram.
 //    Filtered arithmetic: OpenCV's source coordinate is rint() of an f64 expression.  An f32 evaluation (error
 //    << 0.05 px for |coord| < 32768) decides every pixel whose coordinate is not within its error bound of a rounding
-//    boundary -- the integer it rounds to is then provably the same; the rest (~10 %) is collected by ballot
-//    compaction and redone densely with the exact f64 sequence.  A lane owns 4 adjacent destination pixels per
+//    boundary -- the integer it rounds to is then provably the same; the rest (a few % on tilted markers) is collected
+//    by ballot compaction and redone densely with the exact f64 sequence.  A lane owns 4 adjacent destination pixels per
 //    step: their 4 gathers are in flight together (r1k: 23 % of the stall samples sat on the single gather) and
 //    the canonical image is written as 32-bit words.
 // ---------------------------------------------------------------------------------------------------
@@ -195,7 +195,9 @@ __global__ void __launch_bounds__(32 * DECODE_WARPS) k_sample(Batch b) {
                         const int i = i0 + 4 * lane + u;
                         if (pos < DECODE_LIST) {
                             s_list[pos] = (unsigned short)i;
-                        } else {  // list full (cannot happen unless the map is degenerate): do it now
+                        } else {  // list full: do it now.  Ordinary quads fill the list: an axis-aligned side of an odd
+                                  // multiple of (S-1)/2 puts every other sample row and column on a half pixel and defers
+                                  // 3/4 of the S*S pixels, more than DECODE_LIST from S = 37 on
                             const int y = i / S, x = i - y * S;
                             int sx, sy;
                             warp_src_coord(ax->Mi, x, y, bw, &sx, &sy);

@@ -358,8 +358,10 @@ class MarkerDetector:
         return q[ids < 0]
 
     def getCanonical(self, frame: int, candidate: int) -> np.ndarray:
-        S = self._p.warp_size
-        out = np.empty((S, S), np.uint8)
+        """S x S canonical image, S = the warp size the batch ran with (setWarpSize may have changed it since)."""
+        S = C.c_int32()
+        self._check(self._lib.ab_get_canonical_size(self._h, C.byref(S)))
+        out = np.empty((S.value, S.value), np.uint8)
         self._check(self._lib.ab_get_canonical(self._h, frame, candidate, _ptr(out)))
         return out
 

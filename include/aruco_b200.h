@@ -138,7 +138,10 @@ AB_API int ab_get_grey(ab_context* ctx, int frame, uint8_t* dst, size_t dst_stri
 /* every candidate that reached the decoder, in the reference's order (cpp:350): quads = n*8 floats (the
  * corners entering warp), ids (-1 = rejected -> getCandidates h:266), n_rot.                              */
 AB_API int ab_get_candidates(ab_context* ctx, int frame, float* quads, int32_t* ids, int32_t* n_rot, int cap, int32_t* n);
+/* canonical image of a candidate: S*S bytes, S = the warp size the batch ran with (ab_get_canonical_size), which
+ * differs from the current parameters when the warp size was changed after that batch was enqueued            */
 AB_API int ab_get_canonical(ab_context* ctx, int frame, int candidate, uint8_t* dst /* S*S */);
+AB_API int ab_get_canonical_size(ab_context* ctx, int32_t* size);
 AB_API int ab_get_contour(ab_context* ctx, int frame, int candidate, int32_t* xy, int cap_points, int32_t* n);
 /* counters[0]=start candidates [1]=contours kept (min<n<max) [2]=contour points [3]=quads before the
  * too-near filter [4]=candidates [5]=markers (summed over the batch)                                      */
