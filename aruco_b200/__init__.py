@@ -6,7 +6,8 @@ thin host mirror of the reference's operator interface in detector.py.  No CPU f
 from .detector import FiducidalMarkers, HighlyReliableMarkers, Marker, MarkerDetector  # noqa: F401
 from ._lib import ArucoError  # noqa: F401
 from .board import Board, BoardConfiguration, BoardDetector  # noqa: F401
+from .calib import calibrateCamera, calibrateCameras  # noqa: F401
 from . import render  # noqa: F401
 
 __all__ = ["MarkerDetector", "Marker", "FiducidalMarkers", "HighlyReliableMarkers", "ArucoError", "Board",
-           "BoardConfiguration", "BoardDetector"]
+           "BoardConfiguration", "BoardDetector", "calibrateCamera", "calibrateCameras"]

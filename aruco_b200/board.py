@@ -166,3 +166,40 @@ class BoardDetector:
     def fetch(self, n_frames: int, cap_per_frame: int = 256):
         """[(prob, Board, markers)] per frame of the oldest enqueued batch."""
         return self._boards(self._mdetector.fetch(n_frames, cap_per_frame))
+
+    # ---- calibration from detected boards (the reference's utils/aruco_calibration) -----------------------------------------
+    @staticmethod
+    def stack_views(results, BConf: BoardConfiguration, markerSizeMeters: float = -1.0, min_markers: int = 4):
+        """The calibration correspondences of the frames in `results` ((prob, Board, markers) per frame, as detect_batch and
+        fetch return them) that matched at least min_markers markers, stacked as the board stage stacks them
+        (board_select_stack): per matched marker in detection order its 4 configuration corners -- times metres per pixel
+        (markerSizeMeters / |corner 0 - corner 1| of the first marker) for a PIX configuration with a marker size -- and its
+        4 image corners.  Returns (objectPoints, imagePoints): lists of f32 (N, 3) / (N, 2) arrays."""
+        objp = {}
+        for i, corners in zip(BConf.ids, BConf.objPoints):
+            objp.setdefault(int(i), corners)  # the first configuration entry with an id wins
+        mpp = 1.0
+        if BConf.mInfoType == BoardConfiguration.PIX and markerSizeMeters > 0:
+            c = BConf.objPoints[0].astype(np.float32)
+            d = (c[0] - c[1]).astype(np.float64)
+            mpp = float(np.float32(markerSizeMeters)) / float(np.sqrt((d * d).sum()))
+        objs, imgs = [], []
+        for _, board, _ in results:
+            ms = [m for m in board if int(m.id) in objp]
+            if len(ms) < min_markers:
+                continue
+            objs.append(np.concatenate([(objp[int(m.id)].astype(np.float64) * mpp).astype(np.float32) for m in ms]))
+            imgs.append(np.concatenate([np.asarray(m.corners, np.float32).reshape(4, 2) for m in ms]))
+        return objs, imgs
+
+    def calibrate(self, results, imageSize, min_markers: int = 4, raw: bool = False):
+        """cv2.calibrateCamera on the device from the armed board's detections: `results` is the [(prob, Board, markers)] list
+        of detect_batch / fetch.  Frames with fewer than min_markers matched markers are skipped (stack_views).  Returns
+        (rms, K, D, rvecs, tvecs) over the kept frames; with raw=True ((rms, K, D, rvecs, tvecs), objectPoints, imagePoints),
+        the f32 points the device used."""
+        from .calib import calibrateCamera
+        if self._bconf is None:
+            raise ArucoError(_lib.AB_E_STATE, "BoardDetector.calibrate: setParams first")
+        objs, imgs = self.stack_views(results, self._bconf, self._markerSize, min_markers)
+        r = calibrateCamera(objs, imgs, imageSize, detector=self._mdetector)
+        return (r, objs, imgs) if raw else r

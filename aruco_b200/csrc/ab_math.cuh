@@ -981,24 +981,11 @@ AB_HD double pnp_accumulate(const Camera& cam, const double* p, const float* obj
     return PAR::sum(e2);
 }
 
-// obj: N x 3 (a z = const plane), img: N x 2 pixels.  Returns false for degenerate input.
+// Normalised DLT (cv::findHomography, method 0, without its refinement): Hm maps object (X, Y) to the undistorted
+// normalised image point of `cam` (with fx = fy = 1, cx = cy = 0 and zero_D: to the pixel itself), scaled so that
+// Hm[8] = 1.  Mc = the object centroid.  Returns false for degenerate input.
 template <class PAR>
-AB_HD bool solve_pnp_planar_t(const Camera& cam, const float* obj, const float* img, int N, double* rvec, double* tvec) {
-    if (N < 4) return false;
-    // object centroid; the board must lie in a z = const plane (every reference board configuration does)
-    double Mc[3] = {0, 0, 0};
-    for (int n = PAR::first(); n < N; n += PAR::step())
-        for (int c = 0; c < 3; c++) Mc[c] += obj[3 * n + c];
-    for (int c = 0; c < 3; c++) Mc[c] = PAR::sum(Mc[c]) / N;
-    double spread = 0, zdev = 0;
-    for (int n = PAR::first(); n < N; n += PAR::step()) {
-        spread += fabs(obj[3 * n] - Mc[0]) + fabs(obj[3 * n + 1] - Mc[1]);
-        zdev += fabs(obj[3 * n + 2] - Mc[2]);
-    }
-    spread = PAR::sum(spread);
-    zdev = PAR::sum(zdev);
-    if (!(spread > 0) || zdev > 1e-6 * spread) return false;
-    // normalised DLT (cv::findHomography, method 0): object (X,Y) -> normalised image (x,y)
+AB_HD bool planar_homography_t(const Camera& cam, const float* obj, const float* img, int N, const double* Mc, double* Hm) {
     double cM[2] = {Mc[0], Mc[1]}, cm[2] = {0, 0}, sM[2] = {0, 0}, sm[2] = {0, 0};
     for (int n = PAR::first(); n < N; n += PAR::step()) {
         double xn, yn;
@@ -1050,7 +1037,7 @@ AB_HD bool solve_pnp_planar_t(const Camera& cam, const float* obj, const float* 
     // H = invHnorm * H0 * Hnorm2
     double iH[9] = {1. / sm[0], 0, cm[0], 0, 1. / sm[1], cm[1], 0, 0, 1};
     double H2[9] = {sM[0], 0, -cM[0] * sM[0], 0, sM[1], -cM[1] * sM[1], 0, 0, 1};
-    double T[9], Hm[9];
+    double T[9];
     for (int i = 0; i < 3; i++)
         for (int j = 0; j < 3; j++) {
             double q = 0;
@@ -1064,9 +1051,31 @@ AB_HD bool solve_pnp_planar_t(const Camera& cam, const float* obj, const float* 
             Hm[i * 3 + j] = q;
         }
     if (fabs(Hm[8]) < 1e-300) return false;
+    for (int j = 0; j < 9; j++) Hm[j] /= Hm[8];
+    return true;
+}
+
+// obj: N x 3 (a z = const plane), img: N x 2 pixels.  Returns false for degenerate input.
+template <class PAR>
+AB_HD bool solve_pnp_planar_t(const Camera& cam, const float* obj, const float* img, int N, double* rvec, double* tvec) {
+    if (N < 4) return false;
+    // object centroid; the board must lie in a z = const plane (every reference board configuration does)
+    double Mc[3] = {0, 0, 0};
+    for (int n = PAR::first(); n < N; n += PAR::step())
+        for (int c = 0; c < 3; c++) Mc[c] += obj[3 * n + c];
+    for (int c = 0; c < 3; c++) Mc[c] = PAR::sum(Mc[c]) / N;
+    double spread = 0, zdev = 0;
+    for (int n = PAR::first(); n < N; n += PAR::step()) {
+        spread += fabs(obj[3 * n] - Mc[0]) + fabs(obj[3 * n + 1] - Mc[1]);
+        zdev += fabs(obj[3 * n + 2] - Mc[2]);
+    }
+    spread = PAR::sum(spread);
+    zdev = PAR::sum(zdev);
+    if (!(spread > 0) || zdev > 1e-6 * spread) return false;
     // Hm maps ABSOLUTE object (X,Y) (Hnorm2 removes the centroid); the reference maps centred coordinates and
     // adds R*T_transform afterwards -- identical pose
-    for (int j = 0; j < 9; j++) Hm[j] /= Hm[8];
+    double Hm[9];
+    if (!planar_homography_t<PAR>(cam, obj, img, N, Mc, Hm)) return false;
     double h1[3] = {Hm[0], Hm[3], Hm[6]}, h2[3] = {Hm[1], Hm[4], Hm[7]}, h3[3] = {Hm[2], Hm[5], Hm[8]};
     double n1 = sqrt(h1[0] * h1[0] + h1[1] * h1[1] + h1[2] * h1[2]);
     double n2 = sqrt(h2[0] * h2[0] + h2[1] * h2[1] + h2[2] * h2[2]);

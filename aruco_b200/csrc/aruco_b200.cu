@@ -21,6 +21,7 @@
 #include "k_render.cuh"
 #include "k_refine.cuh"
 #include "k_finalize.cuh"
+#include "k_calib.cuh"
 
 using namespace ab;
 
@@ -1759,6 +1760,86 @@ int ab_detect_board(ab_context* ctx, const ab_marker* markers, int n, const ab_b
         board_markers[i] = markers[slots[i]];
         board_markers[i].ssize = out->ssize;
     }
+    return AB_OK;
+}
+
+// cv::calibrateCamera for n_cams cameras: the inputs are packed into one host block (one copy in), k_calibrate runs one CTA
+// per camera, and the results and poses come back in one copy.
+int ab_calibrate_cameras(ab_context* ctx, int n_cams, const ab_calib_camera* cams, ab_calib_result* out, double* rvecs, double* tvecs) {
+    if (!ctx) return AB_E_INVALID;
+    if (n_cams < 0 || n_cams > AB_CALIB_MAX_CAMERAS || (n_cams > 0 && (!cams || !out)))
+        return set_err(ctx, AB_E_INVALID, "ab_calibrate_cameras: bad arguments (need 0 <= n_cams <= %d, cams and out)", AB_CALIB_MAX_CAMERAS);
+    long long views = 0, points = 0;
+    for (int c = 0; c < n_cams; c++) {
+        const ab_calib_camera& k = cams[c];
+        if (k.n_views < 0 || k.n_views > AB_CALIB_MAX_VIEWS || k.width < 0 || k.height < 0 || (k.n_views > 0 && !k.n_points))
+            return set_err(ctx, AB_E_INVALID, "ab_calibrate_cameras: camera %d: bad size or view count (at most %d views)", c, AB_CALIB_MAX_VIEWS);
+        long long np = 0;
+        for (int v = 0; v < k.n_views; v++) {
+            if (k.n_points[v] < 0 || k.n_points[v] > AB_CALIB_MAX_VIEW_POINTS)
+                return set_err(ctx, AB_E_INVALID, "ab_calibrate_cameras: camera %d view %d: %d points (0..%d)", c, v, k.n_points[v],
+                               AB_CALIB_MAX_VIEW_POINTS);
+            np += k.n_points[v];
+        }
+        if (np > 0 && (!k.obj || !k.img)) return set_err(ctx, AB_E_INVALID, "ab_calibrate_cameras: camera %d: NULL points", c);
+        views += k.n_views;
+        points += np;
+    }
+    if (points > (1ll << 30)) return set_err(ctx, AB_E_INVALID, "ab_calibrate_cameras: %lld points in one call (at most 2^30)", points);
+    if (ctx->n_pending) return set_err(ctx, AB_E_STATE, "ab_calibrate_cameras: %d batch(es) in flight, fetch them first", ctx->n_pending);
+    if (n_cams == 0) return AB_OK;
+    cudaSetDevice(ctx->device);
+    // device block: cams | n_points | offset | obj | img | results | poses | workspace
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t off_np = al(sizeof(CalibCamRec) * n_cams), off_of = off_np + al(sizeof(int32_t) * views),
+                 off_obj = off_of + al(sizeof(int32_t) * views), off_img = off_obj + al(sizeof(float) * 3 * points),
+                 in_bytes = off_img + al(sizeof(float) * 2 * points), off_res = in_bytes,
+                 off_pose = off_res + al(sizeof(ab_calib_result) * n_cams), off_ws = off_pose + al(sizeof(double) * 6 * views),
+                 total = off_ws + sizeof(CalibView) * views;
+    std::vector<uint8_t> h(off_ws);
+    CalibCamRec* rec = (CalibCamRec*)h.data();
+    int32_t *np = (int32_t*)(h.data() + off_np), *of = (int32_t*)(h.data() + off_of);
+    float *obj = (float*)(h.data() + off_obj), *img = (float*)(h.data() + off_img);
+    int v0 = 0, p0 = 0;
+    for (int c = 0; c < n_cams; c++) {
+        const ab_calib_camera& k = cams[c];
+        rec[c] = CalibCamRec{k.width, k.height, k.n_views, v0};
+        int n = 0;
+        for (int v = 0; v < k.n_views; v++) {
+            np[v0 + v] = k.n_points[v];
+            of[v0 + v] = p0 + n;
+            n += k.n_points[v];
+        }
+        if (n > 0) {
+            memcpy(obj + 3 * (size_t)p0, k.obj, sizeof(float) * 3 * n);
+            memcpy(img + 2 * (size_t)p0, k.img, sizeof(float) * 2 * n);
+        }
+        v0 += k.n_views;
+        p0 += n;
+    }
+    if (int rc = ensure_scratch(ctx, total)) return rc;
+    uint8_t* base = (uint8_t*)ctx->d_scratch;
+    CK(cudaMemcpyAsync(base, h.data(), in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CalibArgs a;
+    a.cams = (const CalibCamRec*)base;
+    a.n_points = (const int32_t*)(base + off_np);
+    a.offset = (const int32_t*)(base + off_of);
+    a.obj = (const float*)(base + off_obj);
+    a.img = (const float*)(base + off_img);
+    a.out = (ab_calib_result*)(base + off_res);
+    a.poses = (double*)(base + off_pose);
+    a.ws = (CalibView*)(base + off_ws);
+    k_calibrate<<<n_cams, CALIB_THREADS, 0, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h.data(), base + off_res, off_ws - off_res, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    memcpy(out, h.data(), sizeof(ab_calib_result) * n_cams);
+    const double* poses = (const double*)(h.data() + (off_pose - off_res));
+    for (long long v = 0; v < views; v++)
+        for (int i = 0; i < 3; i++) {
+            if (rvecs) rvecs[3 * v + i] = poses[6 * v + i];
+            if (tvecs) tvecs[3 * v + i] = poses[6 * v + 3 + i];
+        }
     return AB_OK;
 }
 

@@ -10,6 +10,7 @@
 #pragma once
 #include <algorithm>
 #include <array>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <fstream>
@@ -482,6 +483,37 @@ public:
         return out;
     }
     float get_repj_err_thres() const { return repj_err_thres_; }
+    // The calibration views of detectBatch's boards (the reference's utils/aruco_calibration): boards with at least min_markers
+    // markers, stacked as the board stage stacks them -- per marker its 4 configuration corners (times metres per pixel for a
+    // PIX configuration with a marker size) and its 4 image corners.
+    void stackViews(const std::vector<Board>& boards, std::vector<std::vector<std::array<float, 3>>>& objPoints,
+                    std::vector<std::vector<Point2f>>& imgPoints, size_t min_markers = 4) const {
+        if (!armed_) throw Exception(AB_E_STATE, "BoardDetector::stackViews: setParams first");
+        double mpp = 1.0;
+        if (conf_.mInfoType == BoardConfiguration::PIX && size_ > 0) {
+            const float* c = conf_.objPoints[0].data();
+            mpp = (double)size_ / std::sqrt((double)(c[0] - c[3]) * (c[0] - c[3]) + (double)(c[1] - c[4]) * (c[1] - c[4]) +
+                                            (double)(c[2] - c[5]) * (c[2] - c[5]));
+        }
+        objPoints.clear();
+        imgPoints.clear();
+        for (const Board& b : boards) {
+            std::vector<std::array<float, 3>> o;
+            std::vector<Point2f> im;
+            for (const Marker& m : b) {
+                const int k = conf_.getIndexOfMarkerId(m.id);
+                if (k < 0 || m.size() != 4) continue;
+                for (int p = 0; p < 4; p++) {
+                    o.push_back({(float)((double)conf_.objPoints[k][3 * p] * mpp), (float)((double)conf_.objPoints[k][3 * p + 1] * mpp),
+                                 (float)((double)conf_.objPoints[k][3 * p + 2] * mpp)});
+                    im.push_back(m[p]);
+                }
+            }
+            if (o.size() < 4 * min_markers) continue;
+            objPoints.push_back(o);
+            imgPoints.push_back(im);
+        }
+    }
     // detect (boarddetector.cpp:90-204): returns the fraction of the board's markers that were found
     float detect(const std::vector<Marker>& detectedMarkers, const BoardConfiguration& conf, Board& out, const CameraParameters& cp,
                  float markerSizeMeters = -1) {
@@ -541,6 +573,42 @@ private:
         for (int i = 0; i < res.n_markers; i++) out.push_back(MarkerDetector::convert(matched[i]));
     }
 };
+
+// cv::calibrateCamera(objectPoints, imagePoints, imageSize, K, D, rvecs, tvecs) with flags 0 on the device (ab_calibrate_cameras):
+// object points on the z = 0 plane.  Returns the rms reprojection error; `out` receives K and D (f32, as CameraParameters holds
+// them) and the image size; rvecs / tvecs (optional) the f64 pose of each view.  Throws on degenerate input.
+inline double calibrateCamera(MarkerDetector& md, const std::vector<std::vector<std::array<float, 3>>>& objPoints,
+                              const std::vector<std::vector<Point2f>>& imgPoints, Size imageSize, CameraParameters& out,
+                              std::vector<std::array<double, 3>>* rvecs = nullptr, std::vector<std::array<double, 3>>* tvecs = nullptr) {
+    if (objPoints.size() != imgPoints.size()) throw Exception(AB_E_INVALID, "calibrateCamera: objPoints and imgPoints differ in size");
+    std::vector<int32_t> n;
+    std::vector<float> obj, img;
+    for (size_t v = 0; v < objPoints.size(); v++) {
+        if (objPoints[v].size() != imgPoints[v].size()) throw Exception(AB_E_INVALID, "calibrateCamera: a view's point counts differ");
+        n.push_back((int32_t)objPoints[v].size());
+        for (size_t i = 0; i < objPoints[v].size(); i++) {
+            obj.insert(obj.end(), objPoints[v][i].begin(), objPoints[v][i].end());
+            img.push_back(imgPoints[v][i].x);
+            img.push_back(imgPoints[v][i].y);
+        }
+    }
+    const ab_calib_camera cam = {imageSize.width, imageSize.height, (int32_t)n.size(), n.data(), obj.data(), img.data()};
+    ab_calib_result res;
+    std::vector<double> r(3 * std::max<size_t>(n.size(), 1)), t(r.size());
+    int rc = ab_calibrate_cameras(md.handle(), 1, &cam, &res, r.data(), t.data());
+    if (rc != AB_OK) throw Exception(rc, ab_last_error(md.handle()));
+    if (res.status != AB_OK) throw Exception(res.status, "calibrateCamera: degenerate input (non-planar object points, fewer than 2 views, "
+                                                         "a view with fewer than 4 points, or views that do not determine the focal lengths)");
+    float K[9], D[5];
+    for (int i = 0; i < 9; i++) K[i] = (float)res.K[i];
+    for (int i = 0; i < 5; i++) D[i] = (float)res.D[i];
+    out.setParams(K, D, imageSize);
+    for (size_t v = 0; v < n.size(); v++) {
+        if (rvecs) rvecs->push_back({r[3 * v], r[3 * v + 1], r[3 * v + 2]});
+        if (tvecs) tvecs->push_back({t[3 * v], t[3 * v + 1], t[3 * v + 2]});
+    }
+    return res.rms;
+}
 
 // ---- HRM dictionary (src/highlyreliablemarkers.h:95-112) -------------------------------------------------------------
 struct Dictionary {

@@ -216,6 +216,36 @@ AB_API int ab_set_board(ab_context* ctx, const ab_board_config* cfg, const float
  * than cap_per_frame.                                                                                                 */
 AB_API int ab_get_boards(ab_context* ctx, int n_frames, ab_board* boards, ab_marker* board_markers, int cap_per_frame);
 
+/* ---- camera calibration from board views: cv::calibrateCamera (flags 0), planar targets ----------------------------------- */
+/* the views of one camera: view v holds n_points[v] correspondences, the views' points stored one after another */
+typedef struct ab_calib_camera {
+    int32_t width, height;         /* imageSize                                 */
+    int32_t n_views;
+    const int32_t* n_points;       /* [n_views]                                 */
+    const float* obj;              /* [sum n_points][3], the z = 0 plane        */
+    const float* img;              /* [sum n_points][2] pixels                  */
+} ab_calib_camera;
+typedef struct ab_calib_result {
+    double K[9];                   /* camera matrix, row-major                  */
+    double D[5];                   /* k1 k2 p1 p2 k3                            */
+    double rms;                    /* sqrt(sum |e|^2 / total points), as cv::calibrateCamera returns it */
+    int32_t iterations;            /* Levenberg-Marquardt iterations (at most 30) */
+    int32_t status;                /* 0, or AB_E_INVALID for a degenerate camera (K, D, rms, poses are then 0) */
+} ab_calib_result;
+/* limits of this implementation (larger inputs return AB_E_INVALID) */
+#define AB_CALIB_MAX_CAMERAS 65536
+#define AB_CALIB_MAX_VIEWS 1024           /* per camera   */
+#define AB_CALIB_MAX_VIEW_POINTS 4096     /* per view     */
+/* Calibrates n_cams cameras in one launch: free parameters fx, fy, cx, cy, k1, k2, p1, p2, k3 and a pose per view; skew, k4..k6,
+ * the thin-prism and tilt terms are 0; termination TermCriteria(COUNT + EPS, 30, DBL_EPSILON).  A camera whose object points
+ * are not in the z = 0 plane (|mean z| or its standard deviation above 1e-5), that has fewer than 2 views, a view with fewer
+ * than 4 points, or views that do not determine the focal lengths (e.g. all parallel to the image plane) gets status
+ * AB_E_INVALID; the other cameras are calibrated and the call returns AB_OK.  rvecs / tvecs ([total views][3] each, in camera
+ * order, may be NULL) receive the pose of each view.  Runs on the context's stream and synchronises; AB_E_STATE while a batch
+ * is in flight.                                                                                                         */
+AB_API int ab_calibrate_cameras(ab_context* ctx, int n_cams, const ab_calib_camera* cams, ab_calib_result* out, double* rvecs,
+                                double* tvecs);
+
 /* ---- next row: marker / board rendering on the device ----------------------------------------------------- */
 /* FiducidalMarkers::createMarkerImage (src/arucofidmarkers.cpp:213-263) without the text watermark (cv::putText
  * glyphs are OpenCV font data: not reproduced, addWaterMark must be false).  The image is square with side
