@@ -25,7 +25,8 @@ oracle/_build/liboracle.so: $(wildcard oracle/*.cpp oracle/*.h)
 	@mkdir -p oracle/_build
 	@if ls oracle/*.cpp >/dev/null 2>&1; then $(CXX) -O2 -fopenmp -ffp-contract=off -shared -fPIC -o $@ oracle/*.cpp; fi
 
-hostcheck: tests/_build/libhostcheck.so tests/_build/libhostcheck_board.so tests/_build/libhostcheck_calib.so
+hostcheck: tests/_build/libhostcheck.so tests/_build/libhostcheck_board.so tests/_build/libhostcheck_calib.so \
+           tests/_build/libhostcheck_stereo.so
 tests/_build/libhostcheck.so: tests/hostcheck/hostcheck.cpp $(wildcard aruco_b200/csrc/*.cuh)
 	@mkdir -p tests/_build
 	$(CXX) -O2 -ffp-contract=off -shared -fPIC -o $@ tests/hostcheck/hostcheck.cpp
@@ -35,11 +36,14 @@ tests/_build/libhostcheck_board.so: tests/hostcheck/hostcheck_board.cpp $(wildca
 tests/_build/libhostcheck_calib.so: tests/hostcheck/hostcheck_calib.cpp $(wildcard aruco_b200/csrc/*.cuh) include/aruco_b200.h
 	@mkdir -p tests/_build
 	$(CXX) -O2 -ffp-contract=off -shared -fPIC -o $@ tests/hostcheck/hostcheck_calib.cpp
+tests/_build/libhostcheck_stereo.so: tests/hostcheck/hostcheck_stereo.cpp $(wildcard aruco_b200/csrc/*.cuh) include/aruco_b200.h
+	@mkdir -p tests/_build
+	$(CXX) -O2 -ffp-contract=off -shared -fPIC -o $@ tests/hostcheck/hostcheck_stereo.cpp
 
 FACADE_HDR := include/aruco/markerdetector.hpp include/aruco/serialization.hpp include/aruco/arucofidmarkers.hpp
 FACADE_LD  := -Laruco_b200/lib -laruco_b200 -Wl,-rpath,'$$ORIGIN/../../aruco_b200/lib'
 facade: tests/_build/aruco_simple tests/_build/aruco_simple_board tests/_build/aruco_create_board tests/_build/yaml_tool tests/_build/aruco_board_batch \
-        tests/_build/aruco_calibration
+        tests/_build/aruco_calibration tests/_build/aruco_stereo_calibration
 tests/_build/%: tests/cpp/%.cpp $(FACADE_HDR) $(LIB)
 	@mkdir -p tests/_build
 	$(CXX) -std=c++14 -O1 -Wall -o $@ $< $(FACADE_LD)

@@ -6,8 +6,10 @@ thin host mirror of the reference's operator interface in detector.py.  No CPU f
 from .detector import FiducidalMarkers, HighlyReliableMarkers, Marker, MarkerDetector  # noqa: F401
 from ._lib import ArucoError  # noqa: F401
 from .board import Board, BoardConfiguration, BoardDetector  # noqa: F401
-from .calib import calibrateCamera, calibrateCameras  # noqa: F401
+from .calib import (CALIB_FIX_INTRINSIC, calibrateCamera, calibrateCameras, stereoCalibrate, stereoCalibrateExtended,  # noqa: F401
+                    stereoCalibratePairs)
 from . import render  # noqa: F401
 
 __all__ = ["MarkerDetector", "Marker", "FiducidalMarkers", "HighlyReliableMarkers", "ArucoError", "Board",
-           "BoardConfiguration", "BoardDetector", "calibrateCamera", "calibrateCameras"]
+           "BoardConfiguration", "BoardDetector", "calibrateCamera", "calibrateCameras", "CALIB_FIX_INTRINSIC", "stereoCalibrate",
+           "stereoCalibrateExtended", "stereoCalibratePairs"]

@@ -47,6 +47,17 @@ class ab_calib_result(C.Structure):
     _fields_ = [("K", C.c_double * 9), ("D", C.c_double * 5), ("rms", C.c_double), ("iterations", C.c_int32), ("status", C.c_int32)]
 
 
+class ab_stereo_pair(C.Structure):
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("n_views", C.c_int32), ("n_points", C.c_void_p), ("obj", C.c_void_p),
+                ("img1", C.c_void_p), ("img2", C.c_void_p), ("K1", C.c_double * 9), ("D1", C.c_double * 5), ("K2", C.c_double * 9),
+                ("D2", C.c_double * 5)]
+
+
+class ab_stereo_result(C.Structure):
+    _fields_ = [("R", C.c_double * 9), ("T", C.c_double * 3), ("E", C.c_double * 9), ("F", C.c_double * 9), ("rms", C.c_double),
+                ("iterations", C.c_int32), ("status", C.c_int32)]
+
+
 DECODER_FN = C.CFUNCTYPE(C.c_int, C.POINTER(C.c_uint8), C.c_int, C.POINTER(C.c_int), C.c_void_p)
 
 # every symbol include/aruco_b200.h declares: name -> (restype, argtypes)
@@ -86,6 +97,7 @@ SYMBOLS = {
     "ab_set_board": (_i, [_vp, _vp, _vp, _vp, _f, _f, _i]),
     "ab_get_boards": (_i, [_vp, _i, _vp, _vp, _i]),
     "ab_calibrate_cameras": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "ab_stereo_calibrate": (_i, [_vp, _i, _vp, _i, _d, _vp, _vp, _vp, _vp]),
     "ab_create_marker_image": (_i, [_vp, _i, _i, _i, _vp, _sz, C.POINTER(C.c_int)]),
     "ab_create_board_image": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _i, _vp, _sz, C.POINTER(C.c_int), C.POINTER(C.c_int), _vp, _vp, _i,
                                    C.POINTER(C.c_int)]),

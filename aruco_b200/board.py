@@ -203,3 +203,44 @@ class BoardDetector:
         objs, imgs = self.stack_views(results, self._bconf, self._markerSize, min_markers)
         r = calibrateCamera(objs, imgs, imageSize, detector=self._mdetector)
         return (r, objs, imgs) if raw else r
+
+    @staticmethod
+    def stack_stereo_views(results1, results2, BConf: BoardConfiguration, markerSizeMeters: float = -1.0, min_markers: int = 4):
+        """The stereo correspondences of two cameras' detections of the same frames (results1[f] and results2[f], as detect_batch
+        and fetch return them): per frame the configuration markers matched by both cameras, in camera 1's detection order,
+        stacked as stack_views stacks them (4 configuration corners each, times metres per pixel for a PIX configuration with a
+        marker size, and the 4 image corners in each camera).  Frames with fewer than min_markers common markers are skipped.
+        Returns (objectPoints, imagePoints1, imagePoints2): lists of f32 (N, 3) / (N, 2) / (N, 2) arrays."""
+        if len(results1) != len(results2):
+            raise ArucoError(_lib.AB_E_INVALID, "stack_stereo_views: the two cameras have %d and %d frames" % (len(results1), len(results2)))
+        objs, imgs1, imgs2 = [], [], []
+        for (p1, b1, m1), (p2, b2, m2) in zip(results1, results2):
+            in2 = {}
+            for m in b2:
+                in2.setdefault(int(m.id), m)
+            both = Board()
+            other = Board()
+            for m in b1:
+                if int(m.id) in in2 and all(int(x.id) != int(m.id) for x in both):
+                    both.append(m)
+                    other.append(in2[int(m.id)])
+            o, i1 = BoardDetector.stack_views([(p1, both, m1)], BConf, markerSizeMeters, min_markers)
+            if not o:
+                continue
+            _, i2 = BoardDetector.stack_views([(p2, other, m2)], BConf, markerSizeMeters, min_markers)
+            objs.append(o[0])
+            imgs1.append(i1[0])
+            imgs2.append(i2[0])
+        return objs, imgs1, imgs2
+
+    def stereoCalibrate(self, results1, results2, K1, D1, K2, D2, min_markers: int = 4, raw: bool = False,
+                        criteria=(3, 30, 1e-6)):
+        """cv2.stereoCalibrate (CALIB_FIX_INTRINSIC) on the device from the armed board's detections in two cameras' frames
+        (stack_stereo_views).  Returns (rms, K1, D1, K2, D2, R, T, E, F); with raw=True (that tuple, objectPoints, imagePoints1,
+        imagePoints2), the f32 points the device used."""
+        from .calib import stereoCalibrate
+        if self._bconf is None:
+            raise ArucoError(_lib.AB_E_STATE, "BoardDetector.stereoCalibrate: setParams first")
+        objs, i1, i2 = self.stack_stereo_views(results1, results2, self._bconf, self._markerSize, min_markers)
+        r = stereoCalibrate(objs, i1, i2, K1, D1, K2, D2, None, criteria=criteria, detector=self._mdetector)
+        return (r, objs, i1, i2) if raw else r

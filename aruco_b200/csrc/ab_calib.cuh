@@ -105,14 +105,12 @@ AB_HD void chol_solve(const double* L, double* b) {
     }
 }
 
-// Projection of the plane point (X, Y, 0) under intrinsics k and pose (R, t) (cvProjectPoints2 with k1 k2 p1 p2 k3), residual
-// e = projection - (u, v) and, with jac, its derivatives ju / jv with respect to (fx fy cx cy k1 k2 p1 p2 k3 | rvec tvec).
-AB_HD void calib_project(const double* k, const double* R, const double dR[3][9], const double* t, double X, double Y, double u,
-                         double v, bool jac, double* e, double* ju, double* jv) {
+// Projection of the camera-frame point (x, y, z) under intrinsics k (cvProjectPoints2 with k1 k2 p1 p2 k3), residual
+// e = projection - (u, v) and, with jac, its derivatives ju / jv[0..8] with respect to (fx fy cx cy k1 k2 p1 p2 k3) and du / dv
+// with respect to (x, y, z).
+AB_HD void calib_distort(const double* k, double x, double y, double z, double u, double v, bool jac, double* e, double* ju,
+                         double* jv, double* du, double* dv) {
     const double fx = k[0], fy = k[1], cx = k[2], cy = k[3], k1 = k[4], k2 = k[5], p1 = k[6], p2 = k[7], k3 = k[8];
-    double x = R[0] * X + R[1] * Y + t[0];
-    double y = R[3] * X + R[4] * Y + t[1];
-    double z = R[6] * X + R[7] * Y + t[2];
     double iz = z ? 1. / z : 1.;
     double xn = x * iz, yn = y * iz;
     double r2 = xn * xn + yn * yn, r4 = r2 * r2, r6 = r4 * r2;
@@ -131,11 +129,22 @@ AB_HD void calib_project(const double* k, const double* R, const double dR[3][9]
     double dxdy = 2 * xn * yn * dc + 2 * p1 * xn + 2 * p2 * yn;
     double dydy = cdist + 2 * yn * yn * dc + 6 * p1 * yn + 2 * p2 * xn;
     double dxn[3] = {iz, 0, -xn * iz}, dyn[3] = {0, iz, -yn * iz};
-    double du[3], dv[3];
     for (int c = 0; c < 3; c++) {
         du[c] = fx * (dxdx * dxn[c] + dxdy * dyn[c]);
         dv[c] = fy * (dxdy * dxn[c] + dydy * dyn[c]);
     }
+}
+
+// Projection of the plane point (X, Y, 0) under intrinsics k and pose (R, t), residual e = projection - (u, v) and, with jac,
+// its derivatives ju / jv with respect to (fx fy cx cy k1 k2 p1 p2 k3 | rvec tvec).
+AB_HD void calib_project(const double* k, const double* R, const double dR[3][9], const double* t, double X, double Y, double u,
+                         double v, bool jac, double* e, double* ju, double* jv) {
+    double x = R[0] * X + R[1] * Y + t[0];
+    double y = R[3] * X + R[4] * Y + t[1];
+    double z = R[6] * X + R[7] * Y + t[2];
+    double du[3], dv[3];
+    calib_distort(k, x, y, z, u, v, jac, e, ju, jv, du, dv);
+    if (!jac) return;
     for (int q = 0; q < 3; q++) {
         double dX[3] = {dR[q][0] * X + dR[q][1] * Y, dR[q][3] * X + dR[q][4] * Y, dR[q][6] * X + dR[q][7] * Y};
         ju[CALIB_NI + q] = du[0] * dX[0] + du[1] * dX[1] + du[2] * dX[2];
@@ -190,14 +199,15 @@ AB_HD void calib_view_sums(const double* k, const double* p, const float* obj, c
     }
 }
 
-// The view's damped pose block Vd = V with its diagonal scaled by 1 + lambda, factored.
-AB_HD bool calib_view_factor(const CalibView& w, double lambda, double L[36]) {
+// A view's damped pose block Vd = V with its diagonal scaled by 1 + lambda, factored.
+AB_HD bool chol_damped(const double V[6][6], double lambda, double L[36]) {
     double A[36];
     for (int i = 0; i < 6; i++)
-        for (int j = 0; j < 6; j++) A[i * 6 + j] = w.V[i][j];
+        for (int j = 0; j < 6; j++) A[i * 6 + j] = V[i][j];
     for (int i = 0; i < 6; i++) A[i * 6 + i] *= 1. + lambda;
     return chol_factor<6>(A, L);
 }
+AB_HD bool calib_view_factor(const CalibView& w, double lambda, double L[36]) { return chol_damped(w.V, lambda, L); }
 
 // initIntrinsicParams2D's two constraints of one view from its homography H (object plane -> pixels, H[8] = 1) and the
 // principal point (a2, a5): rows = {A00, A01, A10, A11, b0, b1}
@@ -240,6 +250,33 @@ constexpr double CALIB_MIN_FOCAL_CONDITION = 1e-10;
 // degrees).  Views parallel to the image plane leave the focal length free: with noise the estimate wanders to 1e2..1e3 times
 // the image size (cv::calibrateCamera returns such values without complaint); such a camera is reported as degenerate.
 constexpr double CALIB_MAX_FOCAL_RATIO = 100.0;
+
+// CvLevMarq::updateAlt's schedule (lambda = 10^lambdaLg10 from 1e-3; a step that raises the error is retried with lambda ten
+// times larger, up to 1e16; every accepted step lowers lambda tenfold, down to 1e-16), run by every thread of EX.  err: the
+// current |e|^2 (shared); calc_j(): J^T J, J^T e and err at the current parameters; save(): previous parameters = current;
+// step(lambda): current = previous - the damped step, and err at it; rel_change(): |current - previous| / |previous|.  Stops
+// after max_iter accepted steps or when rel_change() < eps; returns the iterations run.
+template <class EX, class CALCJ, class SAVE, class STEP, class REL>
+AB_HD int levmarq_schedule(const double& err, CALCJ calc_j, SAVE save, STEP step, REL rel_change, int max_iter, double eps) {
+    int lambdaLg10 = -3, iters = 0;
+    calc_j();
+    for (;;) {
+        // CALC_J -> step
+        save();
+        const double prevErrNorm = err;
+        EX::sync();
+        for (;;) {
+            step(exp(lambdaLg10 * 2.302585092994046));
+            if (err > prevErrNorm && ++lambdaLg10 <= 16) continue;  // CHECK_ERR: worse, raise lambda and step again
+            break;
+        }
+        lambdaLg10 = lambdaLg10 - 1 > -16 ? lambdaLg10 - 1 : -16;
+        const double rel = rel_change();
+        if (++iters >= max_iter || rel < eps) break;
+        calc_j();
+    }
+    return iters;
+}
 
 // cv::calibrateCamera of one camera.  ws: n_views CalibView records; sh: the camera's shared state.  On return (every thread):
 // sh.status = 0 and sh.k, ws[v].p, sh.e2 hold the result, or sh.status = AB_E_INVALID for degenerate input.  *iters: the
@@ -441,26 +478,15 @@ AB_HD void calibrate_camera_t(const CalibCamera& cam, CalibView* ws, CalibShared
         }
         EX::sync();
     };
-    int lambdaLg10 = -3, iters = 0;
-    calc_j();
-    for (;;) {
-        // CALC_J -> step
+    auto save = [&]() {
         for (int v = EX::warp(); v < nv; v += EX::n_warps())
             if (EX::lane0())
                 for (int j = 0; j < 6; j++) ws[v].prev[j] = ws[v].p[j];
         if (EX::tid() == 0)
             for (int i = 0; i < CALIB_NI; i++) sh.kprev[i] = sh.k[i];
-        const double prevErrNorm = sh.e2;
-        EX::sync();
-        double errNorm;
-        for (;;) {
-            step(exp(lambdaLg10 * 2.302585092994046));
-            errNorm = sh.e2;
-            if (errNorm > prevErrNorm && ++lambdaLg10 <= 16) continue;  // CHECK_ERR: worse, raise lambda and step again
-            break;
-        }
-        lambdaLg10 = lambdaLg10 - 1 > -16 ? lambdaLg10 - 1 : -16;
-        // cvNorm(param, prevParam, CV_RELATIVE_L2) over all parameters
+    };
+    // cvNorm(param, prevParam, CV_RELATIVE_L2) over all parameters
+    auto rel_change = [&]() {
         for (int v = EX::warp(); v < nv; v += EX::n_warps())
             if (EX::lane0()) {
                 double dn = 0, pn = 0;
@@ -486,10 +512,9 @@ AB_HD void calibrate_camera_t(const CalibCamera& cam, CalibView* ws, CalibShared
             sh.pn = pn;
         }
         EX::sync();
-        if (++iters >= CALIB_MAX_ITERS || sqrt(sh.dn) / sqrt(sh.pn) < DBL_EPSILON) break;
-        calc_j();
-    }
-    *iters_out = iters;
+        return sqrt(sh.dn) / sqrt(sh.pn);
+    };
+    *iters_out = levmarq_schedule<EX>(sh.e2, calc_j, save, step, rel_change, CALIB_MAX_ITERS, DBL_EPSILON);
     if (EX::tid() == 0) {
         const double fmax = CALIB_MAX_FOCAL_RATIO * (cam.width > cam.height ? cam.width : cam.height);
         bool ok = calib_finite(sh.e2) && sh.k[0] > 0 && sh.k[1] > 0 && sh.k[0] <= fmax && sh.k[1] <= fmax;

@@ -1843,6 +1843,110 @@ int ab_calibrate_cameras(ab_context* ctx, int n_cams, const ab_calib_camera* cam
     return AB_OK;
 }
 
+// cv::stereoCalibrate (CALIB_FIX_INTRINSIC) for n_pairs camera pairs, laid out as ab_calibrate_cameras: one host block in, one
+// CTA per pair (k_stereo_calibrate), results, poses and per-view errors back in one copy.
+int ab_stereo_calibrate(ab_context* ctx, int n_pairs, const ab_stereo_pair* pairs, int max_iter, double eps, ab_stereo_result* out,
+                        double* rvecs, double* tvecs, double* per_view_errors) {
+    if (!ctx) return AB_E_INVALID;
+    if (n_pairs < 0 || n_pairs > AB_CALIB_MAX_CAMERAS || (n_pairs > 0 && (!pairs || !out)))
+        return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: bad arguments (need 0 <= n_pairs <= %d, pairs and out)", AB_CALIB_MAX_CAMERAS);
+    if (max_iter < 1 || max_iter > 1000 || !(eps >= 0) || !(eps - eps == 0))
+        return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: bad criteria (need 1 <= max_iter <= 1000 and finite eps >= 0)");
+    long long views = 0, points = 0;
+    for (int c = 0; c < n_pairs; c++) {
+        const ab_stereo_pair& k = pairs[c];
+        if (k.n_views < 0 || k.n_views > AB_CALIB_MAX_VIEWS || (k.n_views > 0 && !k.n_points))
+            return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: pair %d: bad view count (at most %d views)", c, AB_CALIB_MAX_VIEWS);
+        for (const double* K : {k.K1, k.K2}) {
+            bool ok = K[0] > 0 && K[4] > 0;
+            for (int i = 0; i < 9; i++) ok = ok && K[i] - K[i] == 0;
+            if (!ok) return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: pair %d: camera matrix not finite or fx, fy <= 0", c);
+        }
+        long long np = 0;
+        for (int v = 0; v < k.n_views; v++) {
+            if (k.n_points[v] < 0 || k.n_points[v] > AB_CALIB_MAX_VIEW_POINTS)
+                return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: pair %d view %d: %d points (0..%d)", c, v, k.n_points[v],
+                               AB_CALIB_MAX_VIEW_POINTS);
+            np += k.n_points[v];
+        }
+        if (np > 0 && (!k.obj || !k.img1 || !k.img2)) return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: pair %d: NULL points", c);
+        views += k.n_views;
+        points += np;
+    }
+    if (points > (1ll << 30)) return set_err(ctx, AB_E_INVALID, "ab_stereo_calibrate: %lld points in one call (at most 2^30)", points);
+    if (ctx->n_pending) return set_err(ctx, AB_E_STATE, "ab_stereo_calibrate: %d batch(es) in flight, fetch them first", ctx->n_pending);
+    if (n_pairs == 0) return AB_OK;
+    cudaSetDevice(ctx->device);
+    // device block: pairs | n_points | offset | obj | img1 | img2 | results | poses | errors | workspace
+    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
+    const size_t off_np = al(sizeof(StereoPairRec) * n_pairs), off_of = off_np + al(sizeof(int32_t) * views),
+                 off_obj = off_of + al(sizeof(int32_t) * views), off_i1 = off_obj + al(sizeof(float) * 3 * points),
+                 off_i2 = off_i1 + al(sizeof(float) * 2 * points), in_bytes = off_i2 + al(sizeof(float) * 2 * points),
+                 off_res = in_bytes, off_pose = off_res + al(sizeof(ab_stereo_result) * n_pairs),
+                 off_err = off_pose + al(sizeof(double) * 6 * views), off_ws = off_err + al(sizeof(double) * 2 * views),
+                 total = off_ws + sizeof(StereoView) * views;
+    std::vector<uint8_t> h(off_ws);
+    StereoPairRec* rec = (StereoPairRec*)h.data();
+    int32_t *np = (int32_t*)(h.data() + off_np), *of = (int32_t*)(h.data() + off_of);
+    float *obj = (float*)(h.data() + off_obj), *i1 = (float*)(h.data() + off_i1), *i2 = (float*)(h.data() + off_i2);
+    int v0 = 0, p0 = 0;
+    for (int c = 0; c < n_pairs; c++) {
+        const ab_stereo_pair& k = pairs[c];
+        StereoPairRec& r = rec[c];
+        r.n_views = k.n_views;
+        r.view0 = v0;
+        memcpy(r.K1, k.K1, sizeof(r.K1));
+        memcpy(r.K2, k.K2, sizeof(r.K2));
+        stereo_intrinsics(k.K1, k.D1, r.kk1);
+        stereo_intrinsics(k.K2, k.D2, r.kk2);
+        int n = 0;
+        for (int v = 0; v < k.n_views; v++) {
+            np[v0 + v] = k.n_points[v];
+            of[v0 + v] = p0 + n;
+            n += k.n_points[v];
+        }
+        if (n > 0) {
+            memcpy(obj + 3 * (size_t)p0, k.obj, sizeof(float) * 3 * n);
+            memcpy(i1 + 2 * (size_t)p0, k.img1, sizeof(float) * 2 * n);
+            memcpy(i2 + 2 * (size_t)p0, k.img2, sizeof(float) * 2 * n);
+        }
+        v0 += k.n_views;
+        p0 += n;
+    }
+    if (int rc = ensure_scratch(ctx, total)) return rc;
+    uint8_t* base = (uint8_t*)ctx->d_scratch;
+    CK(cudaMemcpyAsync(base, h.data(), in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    StereoArgs a;
+    a.pairs = (const StereoPairRec*)base;
+    a.n_points = (const int32_t*)(base + off_np);
+    a.offset = (const int32_t*)(base + off_of);
+    a.obj = (const float*)(base + off_obj);
+    a.img1 = (const float*)(base + off_i1);
+    a.img2 = (const float*)(base + off_i2);
+    a.max_iter = max_iter;
+    a.eps = eps;
+    a.out = (ab_stereo_result*)(base + off_res);
+    a.poses = (double*)(base + off_pose);
+    a.errs = (double*)(base + off_err);
+    a.ws = (StereoView*)(base + off_ws);
+    k_stereo_calibrate<<<n_pairs, CALIB_THREADS, 0, ctx->stream>>>(a);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h.data(), base + off_res, off_ws - off_res, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    memcpy(out, h.data(), sizeof(ab_stereo_result) * n_pairs);
+    const double* poses = (const double*)(h.data() + (off_pose - off_res));
+    const double* errs = (const double*)(h.data() + (off_err - off_res));
+    for (long long v = 0; v < views; v++) {
+        for (int i = 0; i < 3; i++) {
+            if (rvecs) rvecs[3 * v + i] = poses[6 * v + i];
+            if (tvecs) tvecs[3 * v + i] = poses[6 * v + 3 + i];
+        }
+        if (per_view_errors)
+            for (int k = 0; k < 2; k++) per_view_errors[2 * v + k] = errs[2 * v + k];
+    }
+    return AB_OK;
+}
+
 int ab_host_alloc(void** ptr, size_t bytes) {
     if (!ptr) return AB_E_INVALID;
     return cudaMallocHost(ptr, bytes) == cudaSuccess ? AB_OK : AB_E_CUDA;

@@ -4,6 +4,7 @@
 // bit-identical from run to run and whichever cameras share the launch.
 #pragma once
 #include "ab_calib.cuh"
+#include "ab_stereo.cuh"
 
 namespace ab {
 
@@ -58,6 +59,52 @@ __global__ void __launch_bounds__(CALIB_THREADS) k_calibrate(CalibArgs a) {
     long long total = 0;
     for (int v = 0; v < rec.n_views; v++) total += cam.n_points[v];
     r.rms = sqrt(sh.e2 / (double)total);
+}
+
+// k_stereo_calibrate: cv::stereoCalibrate (CALIB_FIX_INTRINSIC) for many camera pairs in one launch, laid out as k_calibrate.
+// The arithmetic is stereo_calibrate_t (ab_stereo.cuh).
+struct StereoPairRec {  // one pair of the launch
+    int n_views;
+    int view0;          // index of its first view in the launch's view arrays
+    double K1[9], K2[9];
+    double kk1[CALIB_NI], kk2[CALIB_NI];
+};
+
+struct StereoArgs {
+    const StereoPairRec* pairs;
+    const int32_t* n_points;  // [views]
+    const int32_t* offset;    // [views]: first point of the view in obj / img1 / img2
+    const float* obj;         // [points][3]
+    const float* img1;        // [points][2]
+    const float* img2;        // [points][2]
+    int max_iter;
+    double eps;
+    StereoView* ws;           // [views]
+    ab_stereo_result* out;    // [pairs]
+    double* poses;            // [views][6]: camera 1's rvec, tvec
+    double* errs;             // [views][2]: per-view errors of camera 1 and camera 2
+};
+
+__global__ void __launch_bounds__(CALIB_THREADS) k_stereo_calibrate(StereoArgs a) {
+    __shared__ StereoShared sh;
+    const StereoPairRec& rec = a.pairs[blockIdx.x];
+    StereoPair pr;
+    pr.n_views = rec.n_views;
+    pr.n_points = a.n_points + rec.view0;
+    pr.offset = a.offset + rec.view0;
+    pr.obj = a.obj;
+    pr.img1 = a.img1;
+    pr.img2 = a.img2;
+    for (int i = 0; i < CALIB_NI; i++) {
+        pr.kk1[i] = rec.kk1[i];
+        pr.kk2[i] = rec.kk2[i];
+    }
+    StereoView* ws = a.ws + rec.view0;
+    int iters = 0;
+    stereo_calibrate_t<CalibCtaExec>(pr, ws, sh, a.max_iter, a.eps, &iters);
+    for (int v = threadIdx.x; v < rec.n_views; v += blockDim.x)
+        stereo_view_result(pr, ws, sh, v, a.poses + 6 * ((size_t)rec.view0 + v), a.errs + 2 * ((size_t)rec.view0 + v));
+    if (threadIdx.x == 0) stereo_result(pr, sh, rec.K1, rec.K2, iters, a.out[blockIdx.x]);
 }
 
 }  // namespace ab

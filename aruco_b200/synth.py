@@ -138,6 +138,75 @@ def camera_for(W: int, H: int):
     return K, D
 
 
+def _board_frame_setup(board: np.ndarray, corners: np.ndarray):
+    """The board's pixel -> centred-coordinate map, its outline and its marker corners in board image pixels."""
+    bh, bw = board.shape
+    ctr = np.array([[1, 0, -(bw // 2)], [0, 1, -(bh // 2)], [0, 0, 1]], np.float64)  # image pixel -> centred board coordinate
+    outline = np.array([[0, 0], [bw - 1, 0], [bw - 1, bh - 1], [0, bh - 1]], np.float64)
+    mk = np.asarray(corners, np.float64)[:, :, :2] + np.array([bw // 2, bh // 2], np.float64)
+    return ctr, outline, mk
+
+
+def _project(Hm, p):
+    q = np.concatenate([p, np.ones(p.shape[:-1] + (1,))], axis=-1) @ Hm.T
+    return q[..., :2] / q[..., 2:3]
+
+
+def _draw_board_pose(rng, K, bh, W, H, max_tilt_deg):
+    """One seeded board pose of warp_board: (R, t) in centred board-pixel units."""
+    tilt, phi = np.radians(rng.uniform(0, max_tilt_deg)), rng.uniform(0, 2 * np.pi)
+    psi = np.radians(rng.uniform(-20, 20))
+    a = np.array([np.cos(phi), np.sin(phi), 0.0])  # in-plane tilt axis (Rodrigues)
+    Ax = np.array([[0, -a[2], a[1]], [a[2], 0, -a[0]], [-a[1], a[0], 0]])
+    Rt = np.eye(3) + np.sin(tilt) * Ax + (1 - np.cos(tilt)) * Ax @ Ax
+    Rz = np.array([[np.cos(psi), -np.sin(psi), 0], [np.sin(psi), np.cos(psi), 0], [0, 0, 1]])
+    R = Rt @ Rz
+    Z = K[0, 0] * bh / (rng.uniform(0.65, 0.8) * H)
+    t = np.array([rng.uniform(-0.12, 0.12) * W * Z / K[0, 0], rng.uniform(-0.06, 0.06) * H * Z / K[0, 0], Z])
+    return R, t
+
+
+def _board_visible(Hm, outline, mk, W, H, min_chain, border):
+    """warp_board's constraints: every board corner `border` inside the frame and every marker's 8-connected outline at least
+    min_chain pixels."""
+    o = _project(Hm, outline)
+    if not ((o[:, 0] >= border * W).all() and (o[:, 0] <= (1 - border) * W).all() and (o[:, 1] >= border * H).all()
+            and (o[:, 1] <= (1 - border) * H).all()):
+        return False
+    q = _project(Hm, mk)
+    d = np.abs(q - np.roll(q, -1, axis=1))
+    return np.max(d, axis=2).sum(axis=1).min() >= min_chain
+
+
+def _render_board(board_f: np.ndarray, Hm: np.ndarray, W: int, H: int, rng, sigma: float) -> np.ndarray:
+    """The board image (f32) under the homography Hm: bilinear sampling with white fill, render_frame's blur and additive
+    Gaussian noise sigma drawn from rng.  Returns the u8 frame."""
+    bh, bw = board_f.shape
+    Hi = np.linalg.inv(Hm)
+    xs = np.arange(W, dtype=np.float64)
+    ys = np.arange(H, dtype=np.float64)[:, None]
+    den = Hi[2, 0] * xs[None, :] + Hi[2, 1] * ys + Hi[2, 2]
+    sx = (Hi[0, 0] * xs[None, :] + Hi[0, 1] * ys + Hi[0, 2]) / den
+    sy = (Hi[1, 0] * xs[None, :] + Hi[1, 1] * ys + Hi[1, 2]) / den
+    fx, fy = np.floor(sx), np.floor(sy)
+    ax, ay = (sx - fx).astype(np.float32), (sy - fy).astype(np.float32)
+    ix, iy = fx.astype(np.int64), fy.astype(np.int64)
+    inside = (ix >= 0) & (iy >= 0) & (ix < bw - 1) & (iy < bh - 1)
+    ixc, iyc = np.clip(ix, 0, bw - 2), np.clip(iy, 0, bh - 2)
+    v = (board_f[iyc, ixc] * (1 - ax) * (1 - ay) + board_f[iyc, ixc + 1] * ax * (1 - ay)
+         + board_f[iyc + 1, ixc] * (1 - ax) * ay + board_f[iyc + 1, ixc + 1] * ax * ay)
+    img = np.where(inside, v, np.float32(255))
+    # the 3x3 Gaussian (sigma 0.8) of render_frame: without it erosion breaks the thin threshold outlines of tilted edges
+    g = np.exp(-1.0 / (2 * 0.8 * 0.8))
+    k3 = np.array([g, 1.0, g], np.float32) / np.float32(1 + 2 * g)
+    p = np.pad(img, 1, mode="edge")
+    img = p[:, :-2] * k3[0] + p[:, 1:-1] * k3[1] + p[:, 2:] * k3[2]
+    img = img[:-2] * k3[0] + img[1:-1] * k3[1] + img[2:] * k3[2]
+    if sigma > 0:
+        img = img + rng.normal(0.0, sigma, size=img.shape).astype(np.float32)
+    return np.clip(np.rint(img), 0, 255).astype(np.uint8)
+
+
 def warp_board(board: np.ndarray, corners: np.ndarray, n_frames: int, W: int, H: int, seed: int, sigma: float = 1.5,
                max_tilt_deg: float = 40.0, min_chain: float = 240.0, border: float = 0.03):
     """n_frames views of a rendered board (u8 image, white background) through the pinhole camera of camera_for(W, H), each
@@ -152,61 +221,51 @@ def warp_board(board: np.ndarray, corners: np.ndarray, n_frames: int, W: int, H:
     bh, bw = board.shape
     K, _ = camera_for(W, H)
     K = K.astype(np.float64)
-    ctr = np.array([[1, 0, -(bw // 2)], [0, 1, -(bh // 2)], [0, 0, 1]], np.float64)  # image pixel -> centred board coordinate
-    outline = np.array([[0, 0], [bw - 1, 0], [bw - 1, bh - 1], [0, bh - 1]], np.float64)
-    mk = np.asarray(corners, np.float64)[:, :, :2] + np.array([bw // 2, bh // 2], np.float64)
-
-    def project(Hm, p):
-        q = np.concatenate([p, np.ones(p.shape[:-1] + (1,))], axis=-1) @ Hm.T
-        return q[..., :2] / q[..., 2:3]
-
+    ctr, outline, mk = _board_frame_setup(board, corners)
     frames = np.empty((n_frames, H, W), np.uint8)
     homs = np.empty((n_frames, 3, 3))
     board_f = board.astype(np.float32)
     for f in range(n_frames):
         for _ in range(1000):
-            tilt, phi = np.radians(rng.uniform(0, max_tilt_deg)), rng.uniform(0, 2 * np.pi)
-            psi = np.radians(rng.uniform(-20, 20))
-            a = np.array([np.cos(phi), np.sin(phi), 0.0])  # in-plane tilt axis (Rodrigues)
-            Ax = np.array([[0, -a[2], a[1]], [a[2], 0, -a[0]], [-a[1], a[0], 0]])
-            Rt = np.eye(3) + np.sin(tilt) * Ax + (1 - np.cos(tilt)) * Ax @ Ax
-            Rz = np.array([[np.cos(psi), -np.sin(psi), 0], [np.sin(psi), np.cos(psi), 0], [0, 0, 1]])
-            R = Rt @ Rz
-            Z = K[0, 0] * bh / (rng.uniform(0.65, 0.8) * H)
-            t = np.array([rng.uniform(-0.12, 0.12) * W * Z / K[0, 0], rng.uniform(-0.06, 0.06) * H * Z / K[0, 0], Z])
+            R, t = _draw_board_pose(rng, K, bh, W, H, max_tilt_deg)
             Hm = K @ np.column_stack([R[:, 0], R[:, 1], t]) @ ctr
-            o = project(Hm, outline)
-            if not ((o[:, 0] >= border * W).all() and (o[:, 0] <= (1 - border) * W).all() and (o[:, 1] >= border * H).all()
-                    and (o[:, 1] <= (1 - border) * H).all()):
-                continue
-            q = project(Hm, mk)
-            d = np.abs(q - np.roll(q, -1, axis=1))
-            if np.max(d, axis=2).sum(axis=1).min() >= min_chain:
+            if _board_visible(Hm, outline, mk, W, H, min_chain, border):
                 break
         else:
             raise RuntimeError("warp_board: no pose satisfies the constraints")
         homs[f] = Hm
-        Hi = np.linalg.inv(Hm)
-        xs = np.arange(W, dtype=np.float64)
-        ys = np.arange(H, dtype=np.float64)[:, None]
-        den = Hi[2, 0] * xs[None, :] + Hi[2, 1] * ys + Hi[2, 2]
-        sx = (Hi[0, 0] * xs[None, :] + Hi[0, 1] * ys + Hi[0, 2]) / den
-        sy = (Hi[1, 0] * xs[None, :] + Hi[1, 1] * ys + Hi[1, 2]) / den
-        fx, fy = np.floor(sx), np.floor(sy)
-        ax, ay = (sx - fx).astype(np.float32), (sy - fy).astype(np.float32)
-        ix, iy = fx.astype(np.int64), fy.astype(np.int64)
-        inside = (ix >= 0) & (iy >= 0) & (ix < bw - 1) & (iy < bh - 1)
-        ixc, iyc = np.clip(ix, 0, bw - 2), np.clip(iy, 0, bh - 2)
-        v = (board_f[iyc, ixc] * (1 - ax) * (1 - ay) + board_f[iyc, ixc + 1] * ax * (1 - ay)
-             + board_f[iyc + 1, ixc] * (1 - ax) * ay + board_f[iyc + 1, ixc + 1] * ax * ay)
-        img = np.where(inside, v, np.float32(255))
-        # the 3x3 Gaussian (sigma 0.8) of render_frame: without it erosion breaks the thin threshold outlines of tilted edges
-        g = np.exp(-1.0 / (2 * 0.8 * 0.8))
-        k3 = np.array([g, 1.0, g], np.float32) / np.float32(1 + 2 * g)
-        p = np.pad(img, 1, mode="edge")
-        img = p[:, :-2] * k3[0] + p[:, 1:-1] * k3[1] + p[:, 2:] * k3[2]
-        img = img[:-2] * k3[0] + img[1:-1] * k3[1] + img[2:] * k3[2]
-        if sigma > 0:
-            img = img + rng.normal(0.0, sigma, size=img.shape).astype(np.float32)
-        frames[f] = np.clip(np.rint(img), 0, 255).astype(np.uint8)
+        frames[f] = _render_board(board_f, Hm, W, H, rng, sigma)
     return frames, homs
+
+
+def warp_board_stereo(board: np.ndarray, corners: np.ndarray, n_frames: int, W: int, H: int, seed: int, R_lr, t_lr, sigma: float = 1.5,
+                      max_tilt_deg: float = 40.0, min_chain: float = 240.0, border: float = 0.03):
+    """n_frames pairs of views of a rendered board by two camera_for(W, H) cameras: camera 2 sees the camera-1 point x as
+    R_lr x + t_lr (t_lr in the units of `corners`, board pixels).  Each frame draws one board pose as warp_board does (pose
+    relative to camera 1) and redraws it until the board satisfies warp_board's border and outline constraints in both
+    frames; both frames are rendered with warp_board's sampling, blur and noise.  Returns (frames1, frames2 u8 [n_frames, H,
+    W], poses [n_frames, 3, 4]: camera 1's [R | t] of the board, in board pixels)."""
+    rng = np.random.default_rng(seed)
+    bh, bw = board.shape
+    K, _ = camera_for(W, H)
+    K = K.astype(np.float64)
+    R_lr, t_lr = np.asarray(R_lr, np.float64).reshape(3, 3), np.asarray(t_lr, np.float64).reshape(3)
+    ctr, outline, mk = _board_frame_setup(board, corners)
+    frames1 = np.empty((n_frames, H, W), np.uint8)
+    frames2 = np.empty((n_frames, H, W), np.uint8)
+    poses = np.empty((n_frames, 3, 4))
+    board_f = board.astype(np.float32)
+    for f in range(n_frames):
+        for _ in range(5000):
+            R, t = _draw_board_pose(rng, K, bh, W, H, max_tilt_deg)
+            R2, t2 = R_lr @ R, R_lr @ t + t_lr
+            H1 = K @ np.column_stack([R[:, 0], R[:, 1], t]) @ ctr
+            H2 = K @ np.column_stack([R2[:, 0], R2[:, 1], t2]) @ ctr
+            if t2[2] > 0 and _board_visible(H1, outline, mk, W, H, min_chain, border) and _board_visible(H2, outline, mk, W, H, min_chain, border):
+                break
+        else:
+            raise RuntimeError("warp_board_stereo: no pose satisfies the constraints in both frames")
+        poses[f] = np.column_stack([R, t])
+        frames1[f] = _render_board(board_f, H1, W, H, rng, sigma)
+        frames2[f] = _render_board(board_f, H2, W, H, rng, sigma)
+    return frames1, frames2, poses

@@ -514,6 +514,39 @@ public:
             imgPoints.push_back(im);
         }
     }
+    // The stereo calibration views of two cameras' detectBatch boards of the same frames (boards1[f] and boards2[f]): per frame
+    // the configuration markers matched by both cameras, in camera 1's detection order (each id once), stacked as stackViews
+    // stacks them; frames with fewer than min_markers common markers are skipped.
+    void stackStereoViews(const std::vector<Board>& boards1, const std::vector<Board>& boards2,
+                          std::vector<std::vector<std::array<float, 3>>>& objPoints, std::vector<std::vector<Point2f>>& imgPoints1,
+                          std::vector<std::vector<Point2f>>& imgPoints2, size_t min_markers = 4) const {
+        if (boards1.size() != boards2.size()) throw Exception(AB_E_INVALID, "BoardDetector::stackStereoViews: the cameras' frame counts differ");
+        objPoints.clear();
+        imgPoints1.clear();
+        imgPoints2.clear();
+        for (size_t f = 0; f < boards1.size(); f++) {
+            Board b1, b2;
+            for (const Marker& m : boards1[f]) {
+                if (conf_.getIndexOfMarkerId(m.id) < 0 || m.size() != 4) continue;
+                bool seen = false;
+                for (const Marker& x : b1) seen = seen || x.id == m.id;
+                const Marker* other = nullptr;
+                for (const Marker& x : boards2[f])
+                    if (!other && x.id == m.id && x.size() == 4) other = &x;
+                if (seen || !other) continue;
+                b1.push_back(m);
+                b2.push_back(*other);
+            }
+            std::vector<std::vector<std::array<float, 3>>> o;
+            std::vector<std::vector<Point2f>> i1, i2;
+            stackViews({b1}, o, i1, min_markers);
+            if (o.empty()) continue;
+            stackViews({b2}, o, i2, min_markers);
+            objPoints.push_back(o[0]);
+            imgPoints1.push_back(i1[0]);
+            imgPoints2.push_back(i2[0]);
+        }
+    }
     // detect (boarddetector.cpp:90-204): returns the fraction of the board's markers that were found
     float detect(const std::vector<Marker>& detectedMarkers, const BoardConfiguration& conf, Board& out, const CameraParameters& cp,
                  float markerSizeMeters = -1) {
@@ -608,6 +641,92 @@ inline double calibrateCamera(MarkerDetector& md, const std::vector<std::vector<
         if (tvecs) tvecs->push_back({t[3 * v], t[3 * v + 1], t[3 * v + 2]});
     }
     return res.rms;
+}
+
+// The result of stereoCalibrate: camera 1 -> camera 2 (x2 = R x1 + T), E = [T]x R, F = K2^-T E K1^-1 (F[8] = 1), row-major.
+struct StereoParameters {
+    double R[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, T[3] = {0, 0, 0}, E[9] = {0}, F[9] = {0};
+    double rms = -1;
+};
+
+// cv::stereoCalibrate(objectPoints, imagePoints1, imagePoints2, K1, D1, K2, D2, size, R, T, E, F, CALIB_FIX_INTRINSIC) on the
+// device (ab_stereo_calibrate): the cameras' f32 K and D are widened to f64 and kept fixed; object points on the z = 0
+// plane; TermCriteria(COUNT + EPS, max_iter, eps).  Returns the rms reprojection error over both cameras.  Throws on
+// degenerate input.
+inline double stereoCalibrate(MarkerDetector& md, const std::vector<std::vector<std::array<float, 3>>>& objPoints,
+                              const std::vector<std::vector<Point2f>>& imgPoints1, const std::vector<std::vector<Point2f>>& imgPoints2,
+                              const CameraParameters& cam1, const CameraParameters& cam2, StereoParameters& out, int max_iter = 30,
+                              double eps = 1e-6) {
+    if (objPoints.size() != imgPoints1.size() || objPoints.size() != imgPoints2.size())
+        throw Exception(AB_E_INVALID, "stereoCalibrate: objPoints, imgPoints1 and imgPoints2 differ in size");
+    if (!cam1.isValid() || !cam2.isValid()) throw Exception(AB_E_INVALID, "stereoCalibrate: both cameras need valid parameters");
+    std::vector<int32_t> n;
+    std::vector<float> obj, i1, i2;
+    for (size_t v = 0; v < objPoints.size(); v++) {
+        if (objPoints[v].size() != imgPoints1[v].size() || objPoints[v].size() != imgPoints2[v].size())
+            throw Exception(AB_E_INVALID, "stereoCalibrate: a view's point counts differ");
+        n.push_back((int32_t)objPoints[v].size());
+        for (size_t i = 0; i < objPoints[v].size(); i++) {
+            obj.insert(obj.end(), objPoints[v][i].begin(), objPoints[v][i].end());
+            i1.push_back(imgPoints1[v][i].x);
+            i1.push_back(imgPoints1[v][i].y);
+            i2.push_back(imgPoints2[v][i].x);
+            i2.push_back(imgPoints2[v][i].y);
+        }
+    }
+    ab_stereo_pair pr;
+    std::memset(&pr, 0, sizeof(pr));
+    pr.width = cam1.CamSize.width;
+    pr.height = cam1.CamSize.height;
+    pr.n_views = (int32_t)n.size();
+    pr.n_points = n.data();
+    pr.obj = obj.data();
+    pr.img1 = i1.data();
+    pr.img2 = i2.data();
+    for (int i = 0; i < 9; i++) {
+        pr.K1[i] = cam1.CameraMatrix[i];
+        pr.K2[i] = cam2.CameraMatrix[i];
+    }
+    for (int i = 0; i < 5; i++) {
+        pr.D1[i] = cam1.Distorsion[i];
+        pr.D2[i] = cam2.Distorsion[i];
+    }
+    ab_stereo_result res;
+    int rc = ab_stereo_calibrate(md.handle(), 1, &pr, max_iter, eps, &res, nullptr, nullptr, nullptr);
+    if (rc != AB_OK) throw Exception(rc, ab_last_error(md.handle()));
+    if (res.status != AB_OK) throw Exception(res.status, "stereoCalibrate: degenerate input (no view, a view with fewer than 4 or collinear "
+                                                         "points, object points off the z = 0 plane, or a pose that is not determined)");
+    for (int i = 0; i < 9; i++) {
+        out.R[i] = res.R[i];
+        out.E[i] = res.E[i];
+        out.F[i] = res.F[i];
+    }
+    for (int i = 0; i < 3; i++) out.T[i] = res.T[i];
+    out.rms = res.rms;
+    return res.rms;
+}
+
+// R, T, E, F as cv::FileStorage writes CV_64F matrices (!!opencv-matrix, dt: d), every value with %.17g so that it reads back
+// exactly; rms as a plain value.
+inline void saveStereoParameters(const StereoParameters& sp, const std::string& path) {
+    std::ostringstream o;
+    auto mat = [&](const char* name, const double* v, int rows, int cols) {
+        o << name << ": !!opencv-matrix\n   rows: " << rows << "\n   cols: " << cols << "\n   dt: d\n   data: [ ";
+        for (int i = 0; i < rows * cols; i++) {
+            char b[40];
+            std::snprintf(b, sizeof b, "%.17g", v[i]);
+            o << b << (i + 1 < rows * cols ? ", " : " ]\n");
+        }
+    };
+    o << "%YAML:1.0\n---\n";
+    mat("R", sp.R, 3, 3);
+    mat("T", sp.T, 3, 1);
+    mat("E", sp.E, 3, 3);
+    mat("F", sp.F, 3, 3);
+    char b[40];
+    std::snprintf(b, sizeof b, "%.17g", sp.rms);
+    o << "rms: " << b << "\n";
+    yaml::write_text(path, o.str());
 }
 
 // ---- HRM dictionary (src/highlyreliablemarkers.h:95-112) -------------------------------------------------------------

@@ -246,6 +246,38 @@ typedef struct ab_calib_result {
 AB_API int ab_calibrate_cameras(ab_context* ctx, int n_cams, const ab_calib_camera* cams, ab_calib_result* out, double* rvecs,
                                 double* tvecs);
 
+/* ---- stereo calibration: cv::stereoCalibrate with CALIB_FIX_INTRINSIC, planar targets ------------------------------------- */
+/* the views of one camera pair: view v holds n_points[v] object points and their images in both cameras */
+typedef struct ab_stereo_pair {
+    int32_t width, height;         /* imageSize (not used: the intrinsics are fixed) */
+    int32_t n_views;
+    const int32_t* n_points;       /* [n_views]                                 */
+    const float* obj;              /* [sum n_points][3], the z = 0 plane        */
+    const float* img1;             /* [sum n_points][2] pixels of camera 1      */
+    const float* img2;             /* [sum n_points][2] pixels of camera 2      */
+    double K1[9], D1[5];           /* camera 1: matrix (row-major; skew unused), k1 k2 p1 p2 k3 */
+    double K2[9], D2[5];           /* camera 2                                  */
+} ab_stereo_pair;
+typedef struct ab_stereo_result {
+    double R[9], T[3];             /* camera 1 -> camera 2: x2 = R x1 + T       */
+    double E[9], F[9];             /* essential [T]x R and fundamental K2^-T E K1^-1 (F[8] = 1) */
+    double rms;                    /* sqrt(sum over both cameras |e|^2 / (2 * points per camera)) */
+    int32_t iterations;            /* Levenberg-Marquardt iterations            */
+    int32_t status;                /* 0, or AB_E_INVALID for a degenerate pair (every output of the pair is then 0) */
+} ab_stereo_result;
+/* Calibrates n_pairs camera pairs in one launch (at most AB_CALIB_MAX_CAMERAS pairs, AB_CALIB_MAX_VIEWS views per pair,
+ * AB_CALIB_MAX_VIEW_POINTS points per view): free parameters the relative pose and camera 1's pose per view; K and D fixed;
+ * termination TermCriteria(COUNT + EPS, max_iter, eps) with 1 <= max_iter <= 1000 and finite eps >= 0 (cv2's default: 30,
+ * 1e-6).  A pair without views, with a view of fewer than 4 points or of collinear points, with object points off the z = 0
+ * plane (|mean z| or its standard deviation above 1e-5), or whose pose initialisation or result is not finite gets status
+ * AB_E_INVALID; the other pairs are calibrated and the call returns AB_OK.  NULL inputs, counts beyond the limits, a K that is
+ * not finite or has fx <= 0 or fy <= 0 and bad criteria return AB_E_INVALID for the whole call.  rvecs / tvecs ([total
+ * views][3] each, in pair order, may be NULL) receive camera 1's pose of each view; per_view_errors ([total views][2], may be
+ * NULL) sqrt(|e|^2 / n_points) of each view in camera 1 and camera 2.  Runs on the context's stream and synchronises;
+ * AB_E_STATE while a batch is in flight.                                                                                   */
+AB_API int ab_stereo_calibrate(ab_context* ctx, int n_pairs, const ab_stereo_pair* pairs, int max_iter, double eps,
+                               ab_stereo_result* out, double* rvecs, double* tvecs, double* per_view_errors);
+
 /* ---- next row: marker / board rendering on the device ----------------------------------------------------- */
 /* FiducidalMarkers::createMarkerImage (src/arucofidmarkers.cpp:213-263) without the text watermark (cv::putText
  * glyphs are OpenCV font data: not reproduced, addWaterMark must be false).  The image is square with side
